@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference algorithm on the host CPU
+    python bench.py --gpus 1 ... --dump-outputs DIR          # also store what the last timed step computed
 
 Workload (BASELINE.json configs[2]): htdemucs (random-init, 4 stems, 41.98 M parameters), one
 synthetic stereo 44.1 kHz track of 64 x 7.8 s segments (overlap 0.25, shifts=0) run through
@@ -146,6 +147,30 @@ def ncu_traffic(label: str, mode: str):
             "source": os.path.relpath(path, ROOT)}
 
 
+DUMP_BYTES = 60 << 20      # --dump-outputs: data in all; with the .npy headers still under 64 MB (10^6 or 2^20 bytes)
+DUMP_WINDOW = 4096         # samples per window of a sampled output
+
+
+def dump_outputs(outdir: str, arrays: dict) -> None:
+    """Write each array of the last timed step as ``<outdir>/<name>.npy`` in float32.  An array larger than its share of
+    DUMP_BYTES keeps the windows of DUMP_WINDOW samples along its last (time) axis at fixed, seeded positions, the same
+    in every run with the same arguments, so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, x in arrays.items():
+        x = x.detach()
+        length = x.shape[-1]
+        if 4 * x.numel() > share:
+            windows = length // DUMP_WINDOW
+            keep = max(1, min(windows, share // (4 * (x.numel() // length) * DUMP_WINDOW)))
+            starts = torch.randperm(windows, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            idx = (starts[:, None] * DUMP_WINDOW + torch.arange(DUMP_WINDOW)).reshape(-1)
+            x = x[..., idx.to(x.device)]
+        np.save(os.path.join(outdir, f"{name}.npy"), x.float().cpu().numpy())
+
+
 def measured_peaks() -> dict:
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -158,7 +183,7 @@ def measured_peaks() -> dict:
 # ------------------------------------------------------------------------------------------ CPU arms
 def cpu_apply_seconds(length: int, reps: int, threads: int, want_output: bool = False):
     """Time the reference algorithm's apply_model on the host CPU: the unmodified reference when
-    its tree is present (build container), else the oracle port (GPU box)."""
+    its tree is present, otherwise the oracle port."""
     import torch
     from oracle import refload
     from demucs_b200.config import htdemucs_config
@@ -199,7 +224,9 @@ def reference_arm(args) -> None:
         return
     threads = os.cpu_count() or 1
     length = CPU_SAMPLE_SEGMENTS * STRIDE
-    times, kind = cpu_apply_seconds(length, args.warmup + args.steps, threads)
+    times, kind, (_, out) = cpu_apply_seconds(length, args.warmup + args.steps, threads, want_output=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stems": out})
     timed = times[args.warmup:]
     sec = sum(timed) / len(timed)
     value = (length / SR) / sec
@@ -279,24 +306,28 @@ def gpu_arm(args) -> None:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            result = None        # free the previous step's output before the next one allocates its own
+            result = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms) / steps
+        return float(ms) / steps, result
 
     for _ in range(max(args.warmup, 3)):
         step_device()
     sampler = ClockSampler(local) if rank == 0 else None
     l0 = sum(e.launches for e in engines)
-    ms = timed(step_device, args.steps)
+    ms, stems = timed(step_device, args.steps)
     launches = torch.tensor([float(sum(e.launches for e in engines) - l0)], device=dev)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stems": stems})
+    del stems
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     from demucs_b200 import apply as _apply
     io = torch.tensor([float(_apply.LAST_IO["h2d_bytes"]), float(_apply.LAST_IO["d2h_bytes"])], dtype=torch.float64,
                       device=dev)      # counted by apply_model from the tensors it copied
@@ -316,7 +347,7 @@ def gpu_arm(args) -> None:
         def step_weak():
             return D.apply_model(model, wmix, device=dev, **kw)
         step_weak()
-        ms_w = timed(step_weak, max(1, args.steps // 2))
+        ms_w, _ = timed(step_weak, max(1, args.steps // 2))
         weak = {"value": (wlen / SR) / (ms_w / 1e3), "unit": UNIT, "ms_per_step": ms_w, "segments_per_gpu": SEGMENTS,
                 "scaling": "weak"}
         del wmix
@@ -453,6 +484,8 @@ def hdemucs_arm(args) -> None:
     ms = timed(step, args.steps)
     launches = eng.launches - l0
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"stems": out})
     step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
     prof = perf.profile_step(eng, step)
@@ -507,7 +540,15 @@ def main():
     ap.add_argument("--batch", type=int, default=64, help="segments per forward (64: one forward per step and GPU, ~36 GB)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / parity leg")
     ap.add_argument("--no-weak", action="store_true", help="N > 1: skip the weak-scaling companion run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the stems of the last one as DIR/stems.npy (float32; beyond "
+                         f"{DUMP_BYTES >> 20} MB, fixed seeded windows of {DUMP_WINDOW} samples along time); "
+                         "the GPU arms need --gpus 1")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1 and args.impl != "reference":
+        ap.error("--dump-outputs needs --gpus 1 (with more, each rank holds only the samples it produced)")
     if args.config == "hdemucs_mmi" and args.impl != "reference":
         return hdemucs_arm(args)
     if args.mode is None:

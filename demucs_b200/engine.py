@@ -253,6 +253,10 @@ class Engine:
 
     def _call(self, name: str, *args) -> None:
         try:
+            # an engine built on a non-CUDA device under the test emulator must not hand host pointers to the CUDA
+            # library once the emulator is gone: on a machine with a GPU the kernels would fault on them
+            if self.device.type != "cuda" and _lib.TEST_HOOK is None:
+                raise _lib.KernelError("demucs_b200 runs on CUDA devices only (there is no CPU path)")
             _lib.call(name, *args)
         except Exception:
             # some workspaces are self-clearing (statistics accumulators, Gram matrices): a forward that dies half-way

@@ -164,6 +164,15 @@ def core_fixture():
     print("core_small", {k: v.shape for k, v in data.items()})
 
 
+def inventory_fixture():
+    """Key order and shapes of the reference's ``HTDemucs.state_dict()`` on the small geometry."""
+    ref = refload.load()
+    sd = ref.HTDemucs(**small_config().reference_kwargs()).state_dict()
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "small_inventory.npz"), names=np.array(list(sd)),
+                        shapes=np.array([str(tuple(v.shape)) for v in sd.values()]))
+    print("small_inventory", len(sd), "tensors")
+
+
 def hdemucs_reference(cfg, W):
     refload.load()
     import demucs.hdemucs as H
@@ -248,6 +257,7 @@ def main():
     forward_fixture("htdemucs_default.npz", full, 0, None, 1, full.segment_length, 29, 4999)
     forward_fixture("htdemucs_ls05.npz", full, 0, 0.5, 1, full.segment_length, 29, 4999)
     apply_fixture()
+    inventory_fixture()
     core_fixture()
     audio_fixture()
     from demucs_b200.hdemucs import hdemucs_mmi_config
