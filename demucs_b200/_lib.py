@@ -13,7 +13,7 @@ import typing as tp
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libdemucs_b200.so")
-SOURCES = ["api.cu", "spectral.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_tc_b16x3.cu", "gemm_tc_b16.cu", "norm.cu", "dconv.cu", "attention.cu", "attention_tc.cu", "attention_b16.cu",
+SOURCES = ["api.cu", "spectral.cu", "gemm_simt.cu", "gemm_tc.cu", "gemm_tc_b16x3.cu", "gemm_tc_b16x3_smem.cu", "gemm_tc_b16.cu", "norm.cu", "dconv.cu", "attention.cu", "attention_tc.cu", "attention_b16.cu",
            "ola.cu", "audio.cu", "hdemucs.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--use_fast_math=false"]

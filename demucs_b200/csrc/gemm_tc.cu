@@ -49,7 +49,8 @@ TileGeom tile_geometry(const bd_gemm_desc& d) {
   return g;
 }
 
-// Tile width of an eligible descriptor.  256-column tiles for the long-K GEMMs whose epilogue has a compile-time
+// Tile width of an eligible descriptor (BD_TC_NO_EXACT is read per call so that both choices can be compared in
+// one process).  256-column tiles for the long-K GEMMs whose epilogue has a compile-time
 // form: one 128x256x8 MMA reads 12 KB of shared memory for the work of two 128x128x8 MMAs (16 KB) -- the tf32
 // kernel is operand-bandwidth-bound -- unless the halved tile count quantises badly over the SMs (short M, N = 512:
 // 2.3 waves instead of 4.5).
@@ -65,7 +66,14 @@ int tile_width(const bd_gemm_desc& d, const TileGeom& g) {
     return (double)t / (double)(((t + 147) / 148) * 148);
   };
   if (wide && wave_eff(256) >= wave_eff(128) - 0.05) return 256;
-  return d.N <= 16 ? 16 : d.N <= 32 ? 32 : d.N <= 64 ? 64 : 128;
+  const int pow2 = d.N <= 16 ? 16 : d.N <= 32 ? 32 : d.N <= 64 ? 64 : 128;
+  // strict mode: 96 / 192-column tiles where the power-of-two ones would pad N by a quarter or more (the N = 96 / 192
+  // decoder and DConv layers: a quarter of the MMAs and B traffic, and for 192 one of two A tile loads, saved)
+  if (d.math == BD_MATH_BF16X3 && getenv("BD_TC_NO_EXACT") == nullptr) {
+    const int exact = (d.N > 64 && d.N <= 96) ? 96 : (d.N > 128 && d.N <= 192) ? 192 : 0;
+    if (exact && wave_eff(exact) >= wave_eff(pow2) - 0.05) return exact;
+  }
+  return pow2;
 }
 
 }  // namespace

@@ -12,11 +12,12 @@
 // running at the same time share the activation rows in L2):
 //   warp 0      TMA producer (one elected lane); the shared-memory ring (4..16 stages) never drains between tiles
 //   warp 1      TMEM allocator + MMA issuer (one elected lane)
-//   warps 4..7  (3xTF32 only) operand splitter: x -> rn_tf32(x), x - rn_tf32(x) in shared memory
+//   warps 4..7  (3xTF32) operand splitter: x -> rn_tf32(x), x - rn_tf32(x) in shared memory (bf16 modes: warps 2..)
 //   last 8..16  epilogue warps, warp w owns TMEM lanes 32*(w%4)..+31.  Wide tiles (TBN >= 64): the 2..4 warps of
 //               a lane quarter split the tile's columns and the accumulator is double-buffered, so the epilogue
-//               of tile i runs under the main loop of tile i+1.  Narrow tiles (TBN <= 32): each group of 4 warps
-//               takes every 4th tile, with 4 accumulators in flight.
+//               of tile i runs under the main loop of tile i+1.  Tiles of 96 / 192 / 256 columns are finished in
+//               chunks of 32 / 64 / 128 so that every warp owns a power-of-two column range.  Narrow tiles
+//               (TBN <= 32): each group of 4 warps takes every 4th tile, with 4 accumulators in flight.
 // The epilogue dumps its TMEM rows into a staging buffer, then walks them with lane = 4-column group so that
 // every global access is a contiguous run of the output row.
 //
@@ -38,10 +39,17 @@
 // gemm_tc.cu / gemm_tc_b16x3.cu / gemm_tc_b16.cu) so that the instantiations build in parallel.
 //   MODE 0  TF32     kind::tf32, single pass
 //   MODE 1  TF32X3   kind::tf32, fp32 hi/lo tiles side by side, 3 products
-//   MODE 2  BF16X3   kind::f16 (bf16): the fp32 A tile is split IN PLACE into bf16 hi / lo tiles by the splitter
-//                    warps, the weights arrive pre-split (bf16 hi / lo planes) by TMA; hi*hi + hi*lo + lo*hi.
+//   MODE 2  BF16X3   kind::f16 (bf16): the splitter warps turn the fp32 A tile into bf16 hi / lo operands, the
+//                    weights arrive pre-split (bf16 hi / lo planes) by TMA; hi*hi + hi*lo + lo*hi.
 //                    16 mantissa bits per operand (rel. error ~4e-6 per layer) at 1.5x the cost of one tf32 pass:
-//                    the arithmetic of the default ("strict", <= 1e-4) mode
+//                    the arithmetic of the default ("strict", <= 1e-4) mode.  The three products of a stage read
+//                    shared memory heavily, so the main loop is bound by its bandwidth (128 B/clk per SM).  Tiles up
+//                    to 192 columns wide (ATM = true) therefore keep the split A operand in TENSOR memory: each
+//                    splitter thread converts one row and stores hi | lo with tcgen05.st into a ring of TBK columns
+//                    per pipeline stage next to the accumulators, and the MMAs read A from there
+//                    (tcgen05.mma [d], [a_tmem], b_desc).  256-column tiles keep the in-place split in shared memory:
+//                    their two accumulators already fill the 512 TMEM columns.  ATM = false is the in-place path
+//                    at every width (BD_TC_SMEM_A=1 selects it, for comparison).
 //   MODE 3  BF16     kind::f16 (bf16), single product (the reduced-precision "bf16" mode)
 //   MODE 4  BF16D    the same with a bf16 A tensor in HBM: the tile arrives by TMA in operand form (64 elements =
 //                    128-byte rows per k-block), no splitter warps
@@ -185,6 +193,15 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem desc], BF16 inputs: A is 128 lanes x 8 columns per K = 16 (two bf16 per column)
+__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout):
 //   [0,14) start>>4 | [16,30) LBO>>4 (unused for swizzled K-major) | [32,46) SBO>>4 = 8 rows * 128 B
@@ -252,6 +269,31 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
         "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
       : "r"(taddr));
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+}
+
+// this thread's TMEM lane, N consecutive 32-bit columns from `taddr`; returns once the data is in tensor memory
+template <int N>
+__device__ __forceinline__ void tmem_st(uint32_t taddr, const uint32_t* r) {
+  static_assert(N == 16 || N == 32, "tmem_st: 16 or 32 columns");
+  if constexpr (N == 32) {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
+        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
+        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+          "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
+          "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
+          "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
+        : "memory");
+  } else {
+    asm volatile(
+        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
+        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
+          "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+        : "memory");
+  }
+  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
 }
 
 // ---- lean epilogue for the common layer shapes -----------------------------------------------------------
@@ -420,8 +462,12 @@ __device__ __forceinline__ int epi_fast_id(const bd_gemm_desc& d, bool vec, bool
 // Epilogue warps per TMEM lane quarter (column split): 4 in the single-pass kernel, where the epilogue is the
 // bottleneck; the 3xTF32 kernel spends 3x longer per tile on the tensor core, so 2 suffice and 4 more warps
 // split the fp32 operand tiles into tf32 hi / lo parts in shared memory.
-template <int TBK, int TBN, int MODE>
+__host__ __device__ constexpr int pow2_at_least(int v, int p) { return p >= v ? p : pow2_at_least(v, 2 * p); }
+
+template <int TBK, int TBN, int MODE, bool ATM = false>
 struct PCfg {
+  static_assert(!ATM || (MODE == BD_TC_BF16X3 && TBN <= 192), "A in tensor memory: strict mode, tiles up to 192 wide");
+  static_assert(TBN % 16 == 0 && TBN <= 256, "UMMA N (M = 128): a multiple of 16 up to 256");
   static constexpr bool kX3 = MODE == BD_TC_TF32X3;                          // fp32 hi / lo tiles side by side
   static constexpr bool kB16 = MODE == BD_TC_BF16X3 || MODE == BD_TC_BF16 || MODE == BD_TC_BF16D;   // bf16 operands
   static constexpr bool kDirect = MODE == BD_TC_BF16D;                       // A is bf16 in HBM
@@ -443,24 +489,32 @@ struct PCfg {
   // (TBN <= 32, the epilogue of one tile is too small to share): each group takes every kPGroups-th TILE
   static constexpr bool kTileSplit = TBN <= 32;
   static constexpr int kNAcc = kTileSplit ? kPGroups : 2;
-  static constexpr int kHalves = TBN > 128 ? 2 : 1;            // 256-column tiles: the epilogue works on 128 at a time
-  static constexpr int kWarpCols = kTileSplit ? TBN : (TBN / kHalves) / kPGroups;
+  // columns the epilogue finishes at a time: every warp of a lane quarter must own a power of two >= 16 of them
+  static constexpr int kChunk = TBN == 256 ? 128 : TBN == 192 ? 64 : TBN == 96 ? 32 : TBN;
+  static constexpr int kChunks = TBN / kChunk;
+  static constexpr int kWarpCols = kTileSplit ? TBN : kChunk / kPGroups;
+  static_assert(kWarpCols >= 16 && (kWarpCols & (kWarpCols - 1)) == 0, "epilogue: power-of-two warp column range");
   static constexpr int kStagingBytes = 4 * kPGroups * 32 * (kWarpCols + 4) * 4;
   static constexpr int kTailBytes = 512 + 128 * kPGroups * 32;   // barriers + TMEM slot, then the row tables
   static constexpr int kBudget = 227 * 1024 - 1024 - kTailBytes - kStagingBytes;
   static constexpr int kStagesRaw = kBudget / (kStageBytesA + kStageBytesB);
   static constexpr int kStages = kStagesRaw > (kTileSplit ? 16 : 8) ? (kTileSplit ? 16 : 8) : kStagesRaw;
   static constexpr int kSmemBytes = kStages * (kStageBytesA + kStageBytesB) + kStagingBytes + 1024 + kTailBytes;
-  static constexpr int kTmemCols = kNAcc * TBN < 32 ? 32 : kNAcc * TBN;
+  // ATM: the A ring in tensor memory has one slot per shared-memory stage (TBK columns = TBK/2 hi + TBK/2 lo, two
+  // bf16 per column) after the accumulators, so the stage's empty barrier also frees its A slot
+  static constexpr int kACol0 = kNAcc * TBN;
+  static constexpr int kTmemUsed = kNAcc * TBN + (ATM ? kStages * TBK : 0);
+  static_assert(kTmemUsed <= 512, "tensor memory: accumulators + A ring exceed 512 columns");
+  static constexpr int kTmemCols = pow2_at_least(kTmemUsed, 32);   // the allocation is a power of two >= 32
 };
 
-template <int TBK, int TBN, int MODE>
-__global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm_tc_persist_kernel(const __grid_constant__ CUtensorMap map_a,
+template <int TBK, int TBN, int MODE, bool ATM>
+__global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv_gemm_tc_persist_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                             const __grid_constant__ CUtensorMap map_b,
                                                                             const __grid_constant__ CUtensorMap map_b_lo,
                                                                             const bd_gemm_desc d, const TileGeom g,
                                                                             int ntiles, int ntn) {
-  using C_ = PCfg<TBK, TBN, MODE>;
+  using C_ = PCfg<TBK, TBN, MODE, ATM>;
   constexpr bool X3 = C_::kX3, B16 = C_::kB16, SPLIT = C_::kSplit;
   constexpr int kPGroups = C_::kPGroups;
   constexpr int kTileBytesA = C_::kTileBytesA, kTileBytesB = C_::kTileBytesB;
@@ -477,7 +531,7 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
   uint64_t* empty_bar = full_bar + kStages;
   constexpr int kNAcc = C_::kNAcc;
   constexpr bool kTileSplit = C_::kTileSplit;
-  constexpr int NH = C_::kHalves;
+  constexpr int NCH = C_::kChunks, CHW = C_::kChunk;
   uint64_t* tmem_full = empty_bar + kStages;       // [kNAcc]
   uint64_t* tmem_empty = tmem_full + kNAcc;        // [kNAcc]
   uint64_t* conv_bar = tmem_empty + kNAcc;             // [kStages] X3: hi/lo tiles written by the splitter warps
@@ -566,7 +620,18 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
           const uint32_t ph = (uint32_t)((kbg / kStages) & 1);
           mbar_wait_parked(SPLIT ? &conv_bar[s] : &full_bar[s], ph);
           tcgen05_fence_after();
-          if constexpr (B16) {
+          if constexpr (ATM) {
+            // A: TMEM slot s = [hi: TBK/2 columns | lo: TBK/2 columns]; B: dense bf16 planes
+            const uint32_t a_hi = tmem_base + (uint32_t)(C_::kACol0 + s * TBK), a_lo = a_hi + TBK / 2;
+            const uint64_t b_hi = make_kmajor_desc16<TBK>(sB + s * kStageBytesB, 8 * TBK * 2);
+            const uint64_t b_lo = make_kmajor_desc16<TBK>(sB + s * kStageBytesB + kTileBytesB, 8 * TBK * 2);
+#pragma unroll
+            for (int k = 0; k < TBK / 16; ++k) {
+              umma_bf16_ts(acc, a_lo + 8 * k, b_hi + 2 * k, idesc, (kb | k) != 0);   // small terms first
+              umma_bf16_ts(acc, a_hi + 8 * k, b_lo + 2 * k, idesc, 1);
+              umma_bf16_ts(acc, a_hi + 8 * k, b_hi + 2 * k, idesc, 1);
+            }
+          } else if constexpr (B16) {
             // A: 8-row groups of [hi 8 x TBK bf16 | lo 8 x TBK bf16] where the fp32 rows were; B: dense bf16 planes
             const uint64_t a_hi = make_kmajor_desc16<TBK>(sA + s * kStageBytesA, C_::kDirect ? 8 * TBK * 2 : 8 * TBK * 4);
             const uint64_t a_lo = make_kmajor_desc16<TBK>(sA + s * kStageBytesA + 8 * TBK * 2, 8 * TBK * 4);
@@ -606,7 +671,39 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
   } else if (SPLIT && warp >= C_::kSplitWarp0 && warp < C_::kSplitWarp0 + C_::kSplitWarps) {
     const int et = threadIdx.x - 32 * C_::kSplitWarp0;      // 0..127
     long long kbg = 0;
-    if constexpr (B16) {
+    if constexpr (ATM) {
+      // ===== operand splitter, A in tensor memory: one thread per tile row =====
+      // Warp w may only touch TMEM lanes 32*(w%4)..+31, so it converts those rows: the thread reads its row's TBK
+      // floats (16-byte chunks in the TMA swizzle: 8 consecutive rows hit 8 different chunk positions, no bank
+      // conflict) and stores bf16 hi | lo into the stage's TMEM slot.  The slot is free once full_bar[s] completes:
+      // the producer refilled stage s only after the MMAs that last read the slot committed empty_bar[s].
+      constexpr int RB = TBK * 4;                          // bytes per fp32 row
+      const int row = 32 * (warp & 3) + lane;
+      const int xr = (row * RB >> 7) & (RB / 16 - 1);      // swizzle XOR term of the row
+      const uint32_t lane_addr = (uint32_t)(32 * (warp & 3)) << 16;
+      (void)et;
+      for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        for (int kb = 0; kb < nkb; ++kb, ++kbg) {
+          const int s = (int)(kbg % kStages);
+          mbar_wait(&full_bar[s], (uint32_t)((kbg / kStages) & 1));
+          const uint8_t* rp = sA + s * kStageBytesA + row * RB;
+          uint32_t hl[TBK];                                // [hi: TBK/2 columns | lo: TBK/2 columns]
+#pragma unroll
+          for (int j = 0; j < TBK / 4; ++j) {
+            const float4 x = *reinterpret_cast<const float4*>(rp + ((j ^ xr) << 4));
+            const uint32_t h0 = pack_bf16(x.x, x.y), h1 = pack_bf16(x.z, x.w);
+            hl[2 * j] = h0;
+            hl[2 * j + 1] = h1;
+            hl[TBK / 2 + 2 * j] = pack_bf16(x.x - __uint_as_float(h0 << 16), x.y - __uint_as_float(h0 & 0xffff0000u));
+            hl[TBK / 2 + 2 * j + 1] = pack_bf16(x.z - __uint_as_float(h1 << 16), x.w - __uint_as_float(h1 & 0xffff0000u));
+          }
+          tcgen05_fence_after();
+          tmem_st<TBK>(tmem_base + lane_addr + (uint32_t)(C_::kACol0 + s * TBK), hl);
+          tcgen05_fence_before();
+          mbar_arrive(&conv_bar[s]);
+        }
+      }
+    } else if constexpr (B16) {
       // ===== operand splitter (bf16 modes): the fp32 A tile becomes bf16 hi (and lo = bf16(x - hi)) IN PLACE =====
       // An 8-row group of the fp32 tile (8 * TBK * 4 bytes, TMA-swizzled) is rewritten as [8 x TBK bf16 hi | 8 x TBK
       // bf16 lo], each half in the K-major swizzle of its own row size.  One warp owns a whole group, so loading the
@@ -737,17 +834,18 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
           asm volatile("prefetch.global.L2 [%0];" ::"l"(pf));
         }
       }
-      // a 256-column tile is finished as two 128-column halves (one staging buffer serves both)
-      for (int half = 0; half < NH; ++half) {
-      const int n0h = n0 + 128 * half;
-      if (half == 0) {
+      // a 96 / 192 / 256-column tile is finished in chunks of CHW columns (one staging buffer serves them all)
+#pragma unroll 1
+      for (int ch = 0; ch < NCH; ++ch) {
+      const int n0h = n0 + CHW * ch;
+      if (ch == 0) {
         mbar_wait_relaxed(&tmem_full[a], (uint32_t)((tcount / kNAcc) & 1));
         tcgen05_fence_after();
       } else {
-        __syncwarp();                              // the staging rows of the first half have been consumed
+        __syncwarp();                              // the staging rows of the previous chunk have been consumed
       }
-      const bool last_half = half == NH - 1;
-      const uint32_t acc = tmem_base + (uint32_t)(a * TBN + 128 * half + cbase) + ((uint32_t)(quarter * 32) << 16);
+      const bool last_chunk = ch == NCH - 1;
+      const uint32_t acc = tmem_base + (uint32_t)(a * TBN + CHW * ch + cbase) + ((uint32_t)(quarter * 32) << 16);
       if (vec) {
         rinfo[lane].obase = er.obase;
         rinfo[lane].i0 = row_ok ? er.i0 : -1;
@@ -766,7 +864,7 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
         }
         tcgen05_fence_before();
         __syncwarp();
-        if (lane == 0 && last_half) mbar_arrive(&tmem_empty[a]);   // accumulator is free for tile i+2 while we finish tile i
+        if (lane == 0 && last_chunk) mbar_arrive(&tmem_empty[a]);   // accumulator is free for tile i+2 while we finish tile i
         if (fast >= 0) {
           const uint32_t st_s = smem_u32(stage), ri_s = smem_u32(rinfo);
           const int n0w = n0h + cbase;
@@ -863,13 +961,13 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE>::kThreads), 1) conv_gemm
         }
         tcgen05_fence_before();
         __syncwarp();
-        if (lane == 0 && last_half) mbar_arrive(&tmem_empty[a]);
-        if (row_stats && row_ok) {
-          atomicAdd(&d.stats_out[2 * (size_t)my_slab], (double)ssum);
-          atomicAdd(&d.stats_out[2 * (size_t)my_slab + 1], (double)ssq);
-        }
+        if (lane == 0 && last_chunk) mbar_arrive(&tmem_empty[a]);
       }
-      }   // half
+      }   // chunk
+      if (!vec && row_stats && row_ok) {       // the row's sums over every chunk
+        atomicAdd(&d.stats_out[2 * (size_t)my_slab], (double)ssum);
+        atomicAdd(&d.stats_out[2 * (size_t)my_slab + 1], (double)ssq);
+      }
       if (d.stats_out && d.stat_mod == 1) {   // one slab per tile (host guarantee): one atomic pair per warp
         const double ds = bd_warp_sum_d((double)ssum), dq = bd_warp_sum_d((double)ssq);
         if (lane == 0) {
@@ -918,9 +1016,9 @@ bool encode(CUtensorMap* map, const void* base, int rank, const cuuint64_t* gdim
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int TBK, int TBN, int MODE>
+template <int TBK, int TBN, int MODE, bool ATM = false>
 int launch_tc_persist(const bd_gemm_desc& d, const TileGeom& g, int items, cudaStream_t st) {
-  using C_ = PCfg<TBK, TBN, MODE>;
+  using C_ = PCfg<TBK, TBN, MODE, ATM>;
   alignas(64) CUtensorMap map_a, map_b, map_b_lo;
   const long long s0 = d.xs_0, s1 = d.J1 > 1 ? d.xs_1 : s0 * d.J0, sb = items > 1 ? d.xs_b : s1 * d.J1;
   constexpr int ES = C_::kDirect ? 2 : 4;            // bytes per element of the A tensor
@@ -961,7 +1059,7 @@ int launch_tc_persist(const bd_gemm_desc& d, const TileGeom& g, int items, cudaS
     return BD_ERR_ARG;
   }
   if (!sms_of[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(conv_gemm_tc_persist_kernel<TBK, TBN, MODE>,
+    cudaError_t e = cudaFuncSetAttribute(conv_gemm_tc_persist_kernel<TBK, TBN, MODE, ATM>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, C_::kSmemBytes);
     if (e != cudaSuccess) {
       bd_set_error("bd_conv_gemm_tc: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
@@ -975,20 +1073,25 @@ int launch_tc_persist(const bd_gemm_desc& d, const TileGeom& g, int items, cudaS
   const int ntn = (d.N + TBN - 1) / TBN;
   const long long ntiles = (long long)items * g.blocks1 * g.blocks0 * ntn;
   const int grid = (int)(ntiles < sms ? ntiles : sms);
-  conv_gemm_tc_persist_kernel<TBK, TBN, MODE><<<grid, C_::kThreads, C_::kSmemBytes, st>>>(map_a, map_b, map_b_lo, d, g,
-                                                                                         (int)ntiles, ntn);
+  conv_gemm_tc_persist_kernel<TBK, TBN, MODE, ATM><<<grid, C_::kThreads, C_::kSmemBytes, st>>>(map_a, map_b, map_b_lo, d,
+                                                                                              g, (int)ntiles, ntn);
   return bd_check_launch("conv_gemm_tc_persist_kernel");
 }
 
-// every tile width of one (k-block depth, arithmetic) pair
-template <int TBK, int MODE>
+// every tile width up to 192 of one (k-block depth, arithmetic, A operand location) triple; the 96 / 192-column
+// tiles exist for the strict mode only (tile_width in gemm_tc.cu)
+template <int TBK, int MODE, bool ATM = false>
 int launch_tc_width(int tbn, const bd_gemm_desc& d, const TileGeom& g, int items, cudaStream_t st) {
   switch (tbn) {
-    case 16: return launch_tc_persist<TBK, 16, MODE>(d, g, items, st);
-    case 32: return launch_tc_persist<TBK, 32, MODE>(d, g, items, st);
-    case 64: return launch_tc_persist<TBK, 64, MODE>(d, g, items, st);
-    case 128: return launch_tc_persist<TBK, 128, MODE>(d, g, items, st);
+    case 16: return launch_tc_persist<TBK, 16, MODE, ATM>(d, g, items, st);
+    case 32: return launch_tc_persist<TBK, 32, MODE, ATM>(d, g, items, st);
+    case 64: return launch_tc_persist<TBK, 64, MODE, ATM>(d, g, items, st);
+    case 128: return launch_tc_persist<TBK, 128, MODE, ATM>(d, g, items, st);
     default: break;
+  }
+  if constexpr (MODE == BD_TC_BF16X3) {
+    if (tbn == 96) return launch_tc_persist<TBK, 96, MODE, ATM>(d, g, items, st);
+    if (tbn == 192) return launch_tc_persist<TBK, 192, MODE, ATM>(d, g, items, st);
   }
   bd_set_error("bd_conv_gemm_tc: no kernel for tile width %d", tbn);
   return BD_ERR_ARG;
