@@ -14,6 +14,7 @@ transposed convolutions read / write contiguous windows, and STFT frames are con
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import math
 import typing as tp
@@ -32,9 +33,10 @@ from .weights import check_state_dict
 # (single bf16 product, <= 1e-2).  "tf32x3" / "tf32" are the kind::tf32 forms of the same two ideas, "fp32" runs the
 # contractions on CUDA cores.
 MODES = ("fp32", "tf32", "tf32x3", "strict", "bf16")
-_GEMM_MATH = {"fp32": _lib.MATH_FP32, "tf32": _lib.MATH_TF32, "tf32x3": _lib.MATH_TF32X3, "strict": _lib.MATH_BF16X3,
-              "bf16": _lib.MATH_BF16}
-_ATTN_MATH = dict(_GEMM_MATH)
+# arithmetic of every contraction of a mode: the implicit GEMM, the attention core and the register-level (mma.sync)
+# thin-layer kernels (single pass, or hi/lo split operands with three products); "fp32" runs them on CUDA cores
+_MATH = {"fp32": _lib.MATH_FP32, "tf32": _lib.MATH_TF32, "tf32x3": _lib.MATH_TF32X3, "strict": _lib.MATH_BF16X3,
+         "bf16": _lib.MATH_BF16}
 
 
 def _interleave_glu(w: torch.Tensor) -> torch.Tensor:
@@ -130,6 +132,46 @@ def pack_dconv(put, packed, state, prefix: str, depth: int, tc_forms: bool, idx=
             put(f"{p}.w2p", pad_rows(packed[f"{p}.w2"].cpu().t()).t())
 
 
+def pack_encoder(put, state, p: str) -> None:
+    """HEncLayer ``p`` (hdemucs.py:123-157): the strided conv tap-major, the k=1 rewrite with its GLU pairs interleaved."""
+    put(f"{p}.conv.w", conv_w(state[f"{p}.conv.weight"]))
+    put(f"{p}.conv.b", state[f"{p}.conv.bias"])
+    put(f"{p}.rewrite.w", _interleave_glu(conv_w(state[f"{p}.rewrite.weight"])))
+    put(f"{p}.rewrite.b", _interleave_glu(state[f"{p}.rewrite.bias"].detach().float()))
+
+
+def pack_decoder(put, state, p: str, tc_forms: bool) -> None:
+    """HDecLayer ``p`` (hdemucs.py:304-335): the rewrite with its GLU pairs interleaved, the k=8 / s=4 transposed conv in
+    its 2-tap form (and the 3-tap tensor-core form), its bias repeated for the 4 output phases of a row."""
+    put(f"{p}.rewrite.w", _interleave_glu(conv_w(state[f"{p}.rewrite.weight"])))
+    put(f"{p}.rewrite.b", _interleave_glu(state[f"{p}.rewrite.bias"].detach().float()))
+    put(f"{p}.conv_tr.w", convtr_w(state[f"{p}.conv_tr.weight"]))
+    if tc_forms:
+        put(f"{p}.conv_tr.w3", convtr_w3(state[f"{p}.conv_tr.weight"]))
+    put(f"{p}.conv_tr.b", state[f"{p}.conv_tr.bias"].detach().float().repeat(4))
+
+
+def _pitch(n: int) -> int:
+    """Item pitch of a time-branch skip tensor: rows padded to a multiple of 4 (zero rows).  That is the reference's own
+    right-padding (hdemucs.py:132-135) and lets the next layer's stride-4 window be a (pos/4, pos%4) TMA box."""
+    return (n + 3) // 4 * 4
+
+
+def _tap(taps, name: str, t: torch.Tensor, fmt: str) -> None:
+    """Record an intermediate in the reference's layout: [B,T,F,C] -> [B,C,F,T] ("f"), [B,T,C] -> [B,C,T] ("t")."""
+    if taps is not None:
+        taps[name] = (t.permute(0, 3, 2, 1) if fmt == "f" else t.permute(0, 2, 1)).clone()
+
+
+def _conv3_geometry(T: int, Fr: int, C_: int, hp: int, dil: int) -> dict:
+    """Implicit-GEMM geometry of the DConv's dilated k=3 conv over T, x [B, T, Fr, C] -> h [B, T, Fr, hp]: positions are
+    the fast axis on the time branch (Fr = 1); on the frequency branch the conv runs along T, the slow axis."""
+    if Fr == 1:
+        return dict(taps=((0, -dil), (0, 0), (0, dil)), I1=1, I0=T, J1=1, J0=T, xs=(T * C_, 0, C_, 1), os_=(T * hp, 0, hp))
+    return dict(taps=((-dil, 0), (0, 0), (dil, 0)), I1=T, I0=Fr, J1=T, J0=Fr,
+                xs=(T * Fr * C_, Fr * C_, C_, 1), os_=(T * Fr * hp, Fr * hp, hp))
+
+
 class PackedWeights:
     """Reference state_dict -> kernel layouts (one-time, on the device)."""
 
@@ -141,28 +183,15 @@ class PackedWeights:
         def put(name, tensor):
             self.t[name] = tensor.detach().to(device=dev, dtype=torch.float32).contiguous()
 
-        def dconv(prefix):
-            pack_dconv(put, self.t, state, prefix, cfg.dconv_depth, tc_forms)
-
         for i in range(cfg.depth):
             for name in ("encoder", "tencoder"):
-                p = f"{name}.{i}"
-                put(f"{p}.conv.w", conv_w(state[f"{p}.conv.weight"]))
-                put(f"{p}.conv.b", state[f"{p}.conv.bias"])
-                put(f"{p}.rewrite.w", _interleave_glu(conv_w(state[f"{p}.rewrite.weight"])))
-                put(f"{p}.rewrite.b", _interleave_glu(state[f"{p}.rewrite.bias"].detach().float()))
+                pack_encoder(put, state, f"{name}.{i}")
                 if cfg.dconv_mode & 1:
-                    dconv(p)
+                    pack_dconv(put, self.t, state, f"{name}.{i}", cfg.dconv_depth, tc_forms)
             for name in ("decoder", "tdecoder"):
-                p = f"{name}.{i}"
-                put(f"{p}.rewrite.w", _interleave_glu(conv_w(state[f"{p}.rewrite.weight"])))
-                put(f"{p}.rewrite.b", _interleave_glu(state[f"{p}.rewrite.bias"].detach().float()))
-                put(f"{p}.conv_tr.w", convtr_w(state[f"{p}.conv_tr.weight"]))
-                if tc_forms:
-                    put(f"{p}.conv_tr.w3", convtr_w3(state[f"{p}.conv_tr.weight"]))
-                put(f"{p}.conv_tr.b", state[f"{p}.conv_tr.bias"].detach().float().repeat(4))
+                pack_decoder(put, state, f"{name}.{i}", tc_forms)
                 if cfg.dconv_mode & 2:
-                    dconv(p)
+                    pack_dconv(put, self.t, state, f"{name}.{i}", cfg.dconv_depth, tc_forms)
         if cfg.freq_emb:
             # x + freq_emb_scale * (emb_scale * E[fr, c])  (htdemucs.py:577-582, hdemucs.py:60-66)
             put("freq_emb", cfg.freq_emb * cfg.emb_scale * state["freq_emb.embedding.weight"].detach().float())
@@ -185,6 +214,8 @@ class PackedWeights:
 class Engine:
     """One HTDemucs model resident on one GPU."""
 
+    Weights = PackedWeights      # state_dict -> kernel layouts; HDemucsEngine packs the v3 state_dict instead
+
     def __init__(self, cfg: HTDemucsConfig, state: tp.Mapping[str, torch.Tensor], device="cuda", mode: str = "fp32"):
         cfg.validate()
         if mode not in MODES:
@@ -195,7 +226,7 @@ class Engine:
         if self.device.type != "cuda" and _lib.TEST_HOOK is None:
             raise _lib.KernelError("demucs_b200 runs on CUDA devices only (there is no CPU path)")
         _lib.lib()  # fail loudly now if the extension is missing
-        self.W = PackedWeights(cfg, state, self.device, tc_forms=(mode != "fp32"))
+        self.W = self.Weights(cfg, state, self.device, tc_forms=(mode != "fp32"))
         # periodic Hann window and twiddles: computed in float64 and rounded once (torch.hann_window in float32 was
         # seen to come back ~3e-5 off on some runs of the same host, which is visible at the 1e-5 STFT tolerance)
         k = np.arange(cfg.nfft, dtype=np.float64)
@@ -203,10 +234,7 @@ class Engine:
         tw = np.stack([np.cos(2 * np.pi * k / cfg.nfft), -np.sin(2 * np.pi * k / cfg.nfft)], axis=1)
         self.twiddle = torch.from_numpy(tw.astype(np.float32)).to(self.device).contiguous()
         self.single_pass = mode in ("tf32", "bf16")      # reduced-precision modes: single-pass mma.sync thin-layer kernels
-        # arithmetic of the register-level (mma.sync) thin-layer kernels: single pass, or hi/lo split operands with
-        # three products in the strict tensor-core modes; the fp32 mode does not use them
-        self.thin_math = {"tf32": _lib.MATH_TF32, "bf16": _lib.MATH_BF16, "tf32x3": _lib.MATH_TF32X3,
-                          "strict": _lib.MATH_BF16X3}.get(mode)
+        self.math = _MATH[mode]
         self._w16_cache: tp.Dict[tp.Tuple, tp.Tuple[torch.Tensor, torch.Tensor]] = {}
         self._bufs: tp.Dict[tp.Tuple, tp.Dict[str, torch.Tensor]] = {}
         self._pos: tp.Dict[tp.Tuple, torch.Tensor] = {}
@@ -304,7 +332,7 @@ class Engine:
         d.stat_div, d.stat_mul, d.stat_mod = stat
         # "bf16" mode: bf16 operands inside the transformer (two thirds of the flops, all of it in LayerScale'd residual
         # branches), single-pass tf32 for the convolutions of the U-Net, whose activations are the main signal path
-        d.math = _lib.MATH_FP32 if not tc else (_lib.MATH_TF32 if (self.mode == "bf16" and not xf) else _GEMM_MATH[self.mode])
+        d.math = _lib.MATH_FP32 if not tc else (_lib.MATH_TF32 if (self.mode == "bf16" and not xf) else self.math)
         if d.math in (_lib.MATH_BF16X3, _lib.MATH_BF16) and Cin % 16 == 0 and _lib.TEST_HOOK is None:
             hi, lo = self._w16(w)
             d.w16_hi, d.w16_lo = ptr(hi), ptr(lo)
@@ -348,17 +376,11 @@ class Engine:
             # (1) h = conv3_dilated(x) and the GroupNorm statistics of h
             if narrow:
                 self._k("bd_dconv_conv3", ptr(x), ptr(W[f"{p}.w1"]), ptr(W[f"{p}.b1"]), ptr(h), hp, ptr(sums), M, C_, hid,
-                        T * Fr, Fr, dil, self.thin_math, self._stream(), flops=2.0 * M * hid * 3 * C_, nbytes=4.0 * M * (C_ + hid),
+                        T * Fr, Fr, dil, self.math, self._stream(), flops=2.0 * M * hid * 3 * C_, nbytes=4.0 * M * (C_ + hid),
                         label="dconv_conv3_mma", detail=f"M={M} C={C_} hid={hid} dil={dil}")
-            elif Fr == 1:   # time branch: positions are the fast axis, one GroupNorm item per batch item
-                geo = dict(taps=((0, -dil), (0, 0), (0, dil)), I1=1, I0=T, J1=1, J0=T,
-                           xs=(T * C_, 0, C_, 1), os_=(T * hp, 0, hp))
-            else:         # frequency branch [B, T, Fr, C]: the conv runs along T, the slow axis
-                geo = dict(taps=((-dil, 0), (0, 0), (dil, 0)), I1=T, I0=Fr, J1=T, J0=Fr,
-                           xs=(T * Fr * C_, Fr * C_, C_, 1), os_=(T * Fr * hp, Fr * hp, hp))
-            if not narrow:
+            else:
                 self._gemm(M=M, N=hp, Cin=C_, x=x, w=W[f"{p}.w1{sfx}"], bias=W[f"{p}.b1{sfx}"], out=h,
-                           stats_out=sums, stat=stat, tc=tc, **geo)
+                           stats_out=sums, stat=stat, tc=tc, **_conv3_geometry(T, Fr, C_, hp, dil))
             self._k("bd_finalize_group_stats", ptr(sums), ptr(mr1), slabs, float(T * hid), self._stream())
             # (2) statistics of u = conv1x1(gelu(gn(h))) WITHOUT storing u: the expanded [.., 2C] tensor never
             #     touches HBM, both passes recompute it from the 8x narrower h (csrc/dconv.cu)
@@ -383,7 +405,7 @@ class Engine:
             self._k("bd_dconv_expand_update", ptr(h), hp, hid, ptr(mr1), ptr(W[f"{p}.g1"]), ptr(W[f"{p}.be1"]),
                     ptr(W[f"{p}.w2t"]), ptr(W[f"{p}.b2"]), ptr(mr2), ptr(W[f"{p}.g2"]), ptr(W[f"{p}.be2"]),
                     ptr(W[f"{p}.scale"]), ptr(x), M, C_, T * Fr, Fr,
-                    self.thin_math if tc else _lib.MATH_FP32, self._stream(),
+                    self.math, self._stream(),
                     nbytes=4.0 * M * (hid + 2 * C_), flops=4.0 * M * hid * C_, label="dconv_expand_update",
                     detail=f"M={M} C={C_} hid={hid}")
 
@@ -394,16 +416,16 @@ class Engine:
         if self.mode == "bf16":
             return self._attention_block_bf16(key, x, kv_src, Win, bin_, B, Tq, Tk, tag)
         att = self._buf(key, f"att{tag}", B * Tq * D)
-        nws = _lib.call_value("bd_attention_workspace", B, H, Tq, Tk, self._math())
+        nws = _lib.call_value("bd_attention_workspace", B, H, Tq, Tk, self.math)
         ws = self._buf(key, f"att_ws{tag}", nws) if nws else None
         label = "attention_simt" if self.mode == "fp32" else "attention_tc"
         # kernels behind the entry point: + V transpose (+ Q / K splits) / the three bf16 conversions
-        nk = {_lib.MATH_FP32: 1, _lib.MATH_TF32: 2, _lib.MATH_TF32X3: 4, _lib.MATH_BF16X3: 4, _lib.MATH_BF16: 4}[self._math()]
+        nk = {_lib.MATH_FP32: 1, _lib.MATH_TF32: 2, _lib.MATH_TF32X3: 4, _lib.MATH_BF16X3: 4, _lib.MATH_BF16: 4}[self.math]
         if kv_src is None:  # self attention: one packed projection
             qkv = self._buf(key, f"qkv{tag}", B * Tq * 3 * D)
             self._gemm(M=B * Tq, N=3 * D, Cin=D, x=x, w=Win, bias=bin_, out=qkv, xf=True)
             self._k("bd_attention", ptr(qkv), qkv.data_ptr() + 4 * D, qkv.data_ptr() + 8 * D, ptr(att),
-                    B, H, Tq, Tq, 3 * D, 3 * D, 3 * D, D, self._math(), ptr(ws), self._stream(),
+                    B, H, Tq, Tq, 3 * D, 3 * D, 3 * D, D, self.math, ptr(ws), self._stream(),
                     flops=4.0 * B * Tq * Tq * D, nbytes=4.0 * B * Tq * D * 4, label=label, kernels=nk)
         else:
             q = self._buf(key, f"q{tag}", B * Tq * D)
@@ -411,7 +433,7 @@ class Engine:
             self._gemm(M=B * Tq, N=D, Cin=D, x=x, w=Win[:D], bias=bin_[:D], out=q, xf=True)
             self._gemm(M=B * Tk, N=2 * D, Cin=D, x=kv_src, w=Win[D:], bias=bin_[D:], out=kv, xf=True)
             self._k("bd_attention", ptr(q), ptr(kv), kv.data_ptr() + 4 * D, ptr(att),
-                    B, H, Tq, Tk, D, 2 * D, 2 * D, D, self._math(), ptr(ws), self._stream(),
+                    B, H, Tq, Tk, D, 2 * D, 2 * D, D, self.math, ptr(ws), self._stream(),
                     flops=4.0 * B * Tq * Tk * D, nbytes=4.0 * B * (2 * Tq + 2 * Tk) * D, label=label, kernels=nk)
         return att
 
@@ -437,11 +459,6 @@ class Engine:
                     B, H, Tq, Tk, D, 2 * D, 2 * D, D, self._stream(),
                     flops=4.0 * B * Tq * Tk * D, nbytes=2.0 * B * (2 * Tq + 2 * Tk) * D, label="attention_tc")
         return att
-
-    def _math(self) -> int:
-        """Arithmetic of the attention core: tcgen05 in both tensor-core modes (three-pass hi/lo products in
-        "tf32x3"), CUDA cores in "fp32"."""
-        return _ATTN_MATH[self.mode]
 
     def _ln(self, x, y, p: str, M: int, pos=None, period=0):
         D = self.cfg.transformer_dim
@@ -476,20 +493,155 @@ class Engine:
         self._k("bd_group_norm_apply", ptr(x), ptr(mr), ptr(W[f"{p}.norm_out.weight"]),
                 ptr(W[f"{p}.norm_out.bias"]), B, T, D, self._stream(), nbytes=8.0 * B * T * D)
 
+    # ------------------------------------------------------------------ layer steps (shared with HDemucsEngine)
+    def _stft(self, key, mix, taps, mag=None):
+        """K1: STFT + CaC pack of mix [B, A, L] and the normalisation statistics -> (spec [B, T, 2048, 2A], norm).
+        forward_core gives the spectrogram ``mag``: only its statistics (and the mix's) are computed then."""
+        B, A, L = mix.shape
+        T = self.cfg.frames(L)
+        st = self._stream()
+        spec = self._buf(key, "spec", B * T * 2048 * 4)
+        stats = self._buf(key, "item_stats", 4 * B, torch.float64)
+        norm = self._buf(key, "item_norm", 8 * B)
+        stats.zero_()
+        if mag is None:
+            self._k("bd_stft_cac", ptr(mix), ptr(self.window), ptr(self.twiddle), ptr(spec), ptr(stats), B, A, L, st,
+                    nbytes=4.0 * B * (A * L + T * 2048 * 4), flops=2.5 * 4096 * 12 * 2 * B * T)
+        else:
+            spec.view(B, T, 2048, 2 * A).copy_(mag.permute(0, 3, 2, 1))
+            pair = self._buf(key, "core_stats", 4 * B, torch.float64)
+            pair.zero_()
+            self._k("bd_item_stats", ptr(spec), ptr(pair), B, 2 * A * 2048 * T, st, nbytes=4.0 * spec.numel())
+            self._k("bd_item_stats", ptr(mix), pair.data_ptr() + 16 * B, B, A * L, st, nbytes=4.0 * mix.numel())
+            stats.view(B, 4)[:, :2].copy_(pair[:2 * B].view(B, 2))
+            stats.view(B, 4)[:, 2:].copy_(pair[2 * B:].view(B, 2))
+        self._k("bd_finalize_item_norm", ptr(stats), ptr(norm), B, float(4 * 2048 * T), float(A * L), st)
+        _tap(taps, "stft", spec.view(B, T, 2048, 4), "f")
+        return spec, norm
+
+    def _time_encoder(self, key, i, x, y_name, norm, taps, B, Tin, Tout, Cin, Cc, conv_only=False) -> torch.Tensor:
+        """Time-branch HEncLayer i (hdemucs.py:123-157): Conv1d(k=8, s=4, p=2) + GELU of x (for i = 0 the mix, normalised
+        on the fly) into buffer ``y_name``, DConv, k=1 rewrite + GLU into the returned skip tensor ``saved_t{i}``.
+        ``conv_only`` (v3's empty time layer, hdemucs.py:137-143): the conv without activation alone; returns y."""
+        W, p = self.W, f"tencoder.{i}"
+        first = i == 0
+        Tin_p = Tin if first else _pitch(Tin)
+        y = self._buf(key, y_name, B * Tout * Cc)
+        if first and self.mode != "fp32" and Cc == 48 and Cin == 2:     # dedicated mma.sync first-layer kernel
+            self._k("bd_encoder_conv0", ptr(x), 1, norm.data_ptr() + 16, 8, ptr(W[f"{p}.conv.w"]), ptr(W[f"{p}.conv.b"]),
+                    ptr(y), B, 1, Tout, Tin, Cin, Cc, self.math, self._stream(), flops=2.0 * B * Tout * Cc * 8 * Cin,
+                    nbytes=4.0 * B * (Cin * Tin + Tout * Cc), label="encoder_conv0_mma", detail=f"M={B * Tout} cin={Cin}")
+        else:
+            self._gemm(M=B * Tout, N=Cc, Cin=Cin, x=x, w=W[f"{p}.conv.w"], bias=W[f"{p}.conv.b"], out=y,
+                       taps=tuple((0, k - 2) for k in range(8)), I1=1, I0=Tout, m0=4, J1=1, J0=Tin_p,
+                       xs=(Cin * Tin, 0, 1, Tin) if first else (Tin_p * Cin, 0, Cin, 1), os_=(Tout * Cc, 0, Cc),
+                       a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE, a_stats=norm[4:] if first else None,
+                       a_stats_stride=8, act=_lib.ACT_NONE if conv_only else _lib.ACT_GELU)
+        if conv_only:
+            _tap(taps, f"tenc{i}", y.view(B, Tout, Cc), "t")
+            return y
+        if self.cfg.dconv_mode & 1:
+            self._dconv(key, p, y, B, Tout, 1, Cc, "_t")
+        z = self._buf(key, f"saved_t{i}", B * _pitch(Tout) * Cc, zero=True)
+        self._gemm(M=B * Tout, N=2 * Cc, Cin=Cc, x=y, w=W[f"{p}.rewrite.w"], bias=W[f"{p}.rewrite.b"], out=z,
+                   act=_lib.ACT_GLU, I1=1, I0=Tout, J1=1, J0=Tout, xs=(Tout * Cc, 0, Cc, 1), os_=(_pitch(Tout) * Cc, 0, Cc))
+        _tap(taps, f"tenc{i}", z.view(B, _pitch(Tout), Cc)[:, :Tout], "t")
+        return z
+
+    def _freq_encoder(self, key, i, x, y_name, norm, taps, B, T, Fin, Cin, Cc) -> torch.Tensor:
+        """Frequency-branch HEncLayer i: Conv2d(k=(8,1), s=(4,1), p=(2,0)) + GELU of x [B, T, Fin, Cin] into buffer
+        ``y_name``, DConv, k=1 rewrite + GLU (+ freq_emb after layer 0) into the returned skip tensor ``saved_f{i}``."""
+        W, p = self.W, f"encoder.{i}"
+        first = i == 0
+        Fo = Fin // 4
+        y = self._buf(key, y_name, B * T * Fo * Cc)
+        if first and self.mode != "fp32" and Cc == 48 and Cin == 4:     # dedicated mma.sync first-layer kernel
+            self._k("bd_encoder_conv0", ptr(x), 0, ptr(norm), 8, ptr(W[f"{p}.conv.w"]), ptr(W[f"{p}.conv.b"]), ptr(y),
+                    B, T, Fo, Fin, Cin, Cc, self.math, self._stream(), flops=2.0 * B * T * Fo * Cc * 8 * Cin,
+                    nbytes=4.0 * B * T * (Fin * Cin + Fo * Cc), label="encoder_conv0_mma", detail=f"M={B * T * Fo} cin={Cin}")
+        else:
+            self._gemm(M=B * T * Fo, N=Cc, Cin=Cin, x=x, w=W[f"{p}.conv.w"], bias=W[f"{p}.conv.b"], out=y,
+                       taps=tuple((0, k - 2) for k in range(8)), I1=T, I0=Fo, m0=4, J1=T, J0=Fin,
+                       xs=(T * Fin * Cin, Fin * Cin, Cin, 1), os_=(T * Fo * Cc, Fo * Cc, Cc),
+                       a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE, a_stats=norm if first else None,
+                       a_stats_stride=8, act=_lib.ACT_GELU)
+        if self.cfg.dconv_mode & 1:
+            self._dconv(key, p, y, B, T, Fo, Cc, "_f")
+        z = self._buf(key, f"saved_f{i}", B * T * Fo * Cc)
+        emb = W["freq_emb"] if (first and self.cfg.freq_emb) else None
+        self._gemm(M=B * T * Fo, N=2 * Cc, Cin=Cc, x=y, w=W[f"{p}.rewrite.w"], bias=W[f"{p}.rewrite.b"], out=z,
+                   act=_lib.ACT_GLU, rowbias=emb, rowbias_period=Fo if emb is not None else 0)
+        _tap(taps, f"enc{i}", z.view(B, T, Fo, Cc), "f")
+        return z
+
+    def _freq_decoder(self, key, j, x, y_name, out, skip, taps, B, T, Fr, Cc, Cout) -> None:
+        """Frequency-branch HDecLayer j: 3x3 rewrite + GLU of x [B, T, Fr, Cc] into buffer ``y_name`` (hdemucs.py:312-313),
+        DConv, ConvTranspose2d(k=(8,1), s=(4,1)) + crop [2:-2] + GELU + skip into ``out`` (hdemucs.py:326-334).  The last
+        layer (skip None) has no activation and writes source-major [B, T, S, F, 4]: an iSTFT frame is contiguous."""
+        W, p = self.W, f"decoder.{j}"
+        last = skip is None
+        y = self._buf(key, y_name, B * T * Fr * Cc)
+        taps9 = tuple((kt - 1, kf - 1) for kf in range(3) for kt in range(3))
+        self._gemm(M=B * T * Fr, N=2 * Cc, Cin=Cc, x=x, w=W[f"{p}.rewrite.w"], bias=W[f"{p}.rewrite.b"], out=y,
+                   taps=taps9, I1=T, I0=Fr, J1=T, J0=Fr, xs=(T * Fr * Cc, Fr * Cc, Cc, 1), os_=(T * Fr * Cc, Fr * Cc, Cc),
+                   act=_lib.ACT_GLU)
+        if self.cfg.dconv_mode & 2:
+            self._dconv(key, p, y, B, T, Fr, Cc, "_f")
+        three = self.mode != "fp32" and 4 * Cout >= 64   # tensor-core form: no halo row
+        self._gemm(M=B * T * (Fr + (0 if three else 1)), N=4 * Cout, Cin=Cc, x=y,
+                   w=W[f"{p}.conv_tr.w3" if three else f"{p}.conv_tr.w"], bias=W[f"{p}.conv_tr.b"], out=out,
+                   taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=T, I0=Fr + (0 if three else 1),
+                   J1=T, J0=Fr, xs=(T * Fr * Cc, Fr * Cc, Cc, 1),
+                   os_=(T * 4 * Fr * Cout, 4 * Fr * Cout, 4 if last else Cout),
+                   oc_split=4 if last else 0, oc_stride=4 * Fr * 4 if last else 0, convt=2 if three else 1, O0=4 * Fr,
+                   act=_lib.ACT_NONE if last else _lib.ACT_GELU, addend=skip)
+        if taps is not None:
+            if last:   # [B,T,S,F,4] -> [B,T,F,(s j)]
+                S = self.cfg.n_sources
+                _tap(taps, f"dec{j}", out.view(B, T, S, 4 * Fr, 4).permute(0, 1, 3, 2, 4).reshape(B, T, 4 * Fr, Cout), "f")
+            else:
+                _tap(taps, f"dec{j}", (out - skip).view(B, T, 4 * Fr, Cout), "f")
+
+    def _time_decoder(self, key, j, x, y_name, out, skip, taps, B, Tin, Tout, Cc, Cout) -> None:
+        """Time-branch HDecLayer j: k=3 rewrite + GLU of x into buffer ``y_name``, DConv, ConvTranspose1d(k=8, s=4) + crop
+        [2:2+Tout] + GELU + skip into ``out``; the last layer (skip None) has no activation."""
+        W, p = self.W, f"tdecoder.{j}"
+        y = self._buf(key, y_name, B * Tin * Cc)
+        self._gemm(M=B * Tin, N=2 * Cc, Cin=Cc, x=x, w=W[f"{p}.rewrite.w"], bias=W[f"{p}.rewrite.b"], out=y,
+                   taps=((0, -1), (0, 0), (0, 1)), I1=1, I0=Tin, J1=1, J0=Tin, xs=(_pitch(Tin) * Cc, 0, Cc, 1),
+                   os_=(Tin * Cc, 0, Cc), act=_lib.ACT_GLU)
+        if self.cfg.dconv_mode & 2:
+            self._dconv(key, p, y, B, Tin, 1, Cc, "_t")
+        three = self.mode != "fp32" and 4 * Cout >= 64
+        self._gemm(M=B * (Tin + (0 if three else 1)), N=4 * Cout, Cin=Cc, x=y,
+                   w=W[f"{p}.conv_tr.w3" if three else f"{p}.conv_tr.w"], bias=W[f"{p}.conv_tr.b"], out=out,
+                   taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=1, I0=Tin + (0 if three else 1),
+                   J1=1, J0=Tin, xs=(Tin * Cc, 0, Cc, 1), os_=(_pitch(Tout) * Cout, 0, Cout), convt=2 if three else 1,
+                   O0=Tout, act=_lib.ACT_NONE if skip is None else _lib.ACT_GELU, addend=skip)
+        if taps is not None:
+            _tap(taps, f"tdec{j}", (out - skip if skip is not None else out).view(B, _pitch(Tout), Cout)[:, :Tout], "t")
+
+    def _istft(self, xf, xt, norm, out_buf, B, T, L, L0) -> torch.Tensor:
+        """K2: de-normalise the spectrogram branch xf, iSTFT, overlap-add in shared memory, crop to L0 samples, add the
+        time branch xt -> [B, S, A, L0] (written into ``out_buf`` when given)."""
+        S, A = self.cfg.n_sources, self.cfg.audio_channels
+        if out_buf is not None:
+            if out_buf.numel() != B * S * A * L0 or out_buf.dtype != torch.float32 or out_buf.device != self.device \
+                    or not out_buf.is_contiguous():
+                raise ValueError("out must be a contiguous float32 tensor of B*S*C*L elements on the engine's device")
+            out = out_buf.view(B, S, A, L0)
+        else:
+            out = torch.empty(B, S, A, L0, dtype=torch.float32, device=self.device)
+        self._k("bd_istft_ola", ptr(xf), ptr(norm), ptr(self.window), ptr(self.twiddle), ptr(xt), ptr(out),
+                B, S, T, _pitch(L), L0, self._stream(), nbytes=4.0 * B * S * (T * 2048 * 4 + 2 * L + 2 * L0),
+                flops=2.5 * 4096 * 12 * 2 * S * B * T)
+        return out
+
     # ------------------------------------------------------------------ forward
     @torch.no_grad()
     def forward(self, mix: torch.Tensor, taps: tp.Optional[dict] = None, out: tp.Optional[torch.Tensor] = None) -> torch.Tensor:
         """mix [B, 2, L <= segment_length] (fp32, on self.device) -> [B, S, 2, L] (written into ``out`` when given)."""
-        # kernels launch on the CURRENT device: make that the engine's device whatever the caller's is; and any
-        # failure -- not only a kernel error -- may leave the self-clearing statistics workspaces dirty
-        try:
-            if self.device.type == "cuda":
-                with torch.cuda.device(self.device):
-                    return self._forward(mix, taps, out)
-            return self._forward(mix, taps, out)
-        except BaseException:
-            self._bufs.clear()
-            raise
+        return self._run(mix, taps, out)
 
     @torch.no_grad()
     def forward_core(self, mag: torch.Tensor, mix: torch.Tensor) -> tp.Tuple[torch.Tensor, torch.Tensor]:
@@ -499,69 +651,43 @@ class Engine:
         (spec_out [B, S, 2*audio_channels, 2048, T], time_out [B, S, audio_channels, L]), both de-normalised.
         The layout changes at this boundary (NCHW in and out) are plain copies; everything between runs in the
         same kernels as ``forward``."""
+        return self._run(mix, None, None, mag)
+
+    def _run(self, mix: torch.Tensor, *args):
+        # kernels launch on the CURRENT device: make that the engine's device whatever the caller's is; and any
+        # failure -- not only a kernel error -- may leave the self-clearing statistics workspaces dirty
         try:
-            if self.device.type == "cuda":
-                with torch.cuda.device(self.device):
-                    return self._forward(mix, None, None, mag=mag)
-            return self._forward(mix, None, None, mag=mag)
+            if mix.dim() != 3 or mix.shape[1] != self.cfg.audio_channels:
+                raise ValueError(f"expected mix of shape [B, {self.cfg.audio_channels}, L], got {tuple(mix.shape)}")
+            if mix.device != self.device or mix.dtype != torch.float32:
+                raise ValueError("mix must be a float32 tensor on the engine's device")
+            with torch.cuda.device(self.device) if self.device.type == "cuda" else contextlib.nullcontext():
+                return self._forward(mix, *args)
         except BaseException:
             self._bufs.clear()
             raise
 
     def _forward(self, mix: torch.Tensor, taps: tp.Optional[dict], out_buf: tp.Optional[torch.Tensor], mag=None):
         cfg, W = self.cfg, self.W
-        if mix.dim() != 3 or mix.shape[1] != cfg.audio_channels:
-            raise ValueError(f"expected mix of shape [B, {cfg.audio_channels}, L], got {tuple(mix.shape)}")
-        if mix.device != self.device or mix.dtype != torch.float32:
-            raise ValueError("mix must be a float32 tensor on the engine's device")
         B, A, L0 = mix.shape
         L = cfg.segment_length
         if L0 > L:  # htdemucs.py:521-524
             raise ValueError(f"Given length {L0} is longer than training length {L}")
         key = (B, L)
-        st = self._stream()
+        S = cfg.n_sources
+        T = cfg.frames(L)
+        chans = cfg.enc_channels
+        if mag is not None and (L0 != L or tuple(mag.shape) != (B, 2 * A, 2048, T) or mag.device != self.device
+                                or mag.dtype != torch.float32):
+            raise ValueError(f"forward_core expects mag [B, {2 * A}, 2048, {T}] and mix [B, {A}, {L}] (float32, on "
+                             f"the engine's device), got {tuple(mag.shape)} and {tuple(mix.shape)}")
         if L0 < L:  # htdemucs.py:534-537: zero-pad on the right up to the training length
             padded = self._buf(key, "mix_padded", B * A * L).view(B, A, L)
             padded.zero_()
             padded[..., :L0].copy_(mix)
             mix = padded
         mix = mix.contiguous()
-        S = cfg.n_sources
-        T = cfg.frames(L)
-        chans = cfg.enc_channels
-
-        def tp(n):   # time-branch item pitch: rows padded to a multiple of 4
-            return (n + 3) // 4 * 4
-
-        def tap(name, t, fmt):
-            if taps is None:
-                return
-            if fmt == "f":    # [B,T,F,C] -> [B,C,F,T]
-                taps[name] = t.permute(0, 3, 2, 1).clone()
-            else:             # [B,T,C] -> [B,C,T]
-                taps[name] = t.permute(0, 2, 1).clone()
-
-        # ---- K1: STFT + CaC pack + normalisation statistics --------------------------------
-        spec = self._buf(key, "spec", B * T * 2048 * 4)
-        stats = self._buf(key, "item_stats", 4 * B, torch.float64)
-        norm = self._buf(key, "item_norm", 8 * B)
-        stats.zero_()
-        if mag is None:
-            self._k("bd_stft_cac", ptr(mix), ptr(self.window), ptr(self.twiddle), ptr(spec), ptr(stats), B, A, L, st,
-                    nbytes=4.0 * B * (A * L + T * 2048 * 4), flops=2.5 * 4096 * 12 * 2 * B * T)
-        else:       # forward_core: the spectrogram is given; only its statistics (and the mix's) are computed here
-            if L0 != L or tuple(mag.shape) != (B, 2 * A, 2048, T) or mag.device != self.device or mag.dtype != torch.float32:
-                raise ValueError(f"forward_core expects mag [B, {2 * A}, 2048, {T}] and mix [B, {A}, {L}] (float32, on "
-                                 f"the engine's device), got {tuple(mag.shape)} and {tuple(mix.shape)}")
-            spec.view(B, T, 2048, 2 * A).copy_(mag.permute(0, 3, 2, 1))
-            pair = self._buf(key, "core_stats", 4 * B, torch.float64)
-            pair.zero_()
-            self._k("bd_item_stats", ptr(spec), ptr(pair), B, 2 * A * 2048 * T, st, nbytes=4.0 * spec.numel())
-            self._k("bd_item_stats", ptr(mix), pair.data_ptr() + 16 * B, B, A * L, st, nbytes=4.0 * mix.numel())
-            stats.view(B, 4)[:, :2].copy_(pair[:2 * B].view(B, 2))
-            stats.view(B, 4)[:, 2:].copy_(pair[2 * B:].view(B, 2))
-        self._k("bd_finalize_item_norm", ptr(stats), ptr(norm), B, float(4 * 2048 * T), float(A * L), st)
-        tap("stft", spec.view(B, T, 2048, 4), "f")
+        spec, norm = self._stft(key, mix, taps, mag)
 
         # ---- encoders ------------------------------------------------------------------------
         tl = cfg.time_lengths(L)
@@ -569,81 +695,33 @@ class Engine:
         xf, Fin, Cin = spec, 2048, 2 * A
         xt, Cin_t = mix, A
         for i, Cc in enumerate(chans):
-            # time branch: Conv1d(k=8,s=4,p=2) on the right-padded signal -> GELU (hdemucs.py:131-144).
-            # Skip tensors are stored with the item length padded to a multiple of 4 (zero rows): that is the
-            # reference's own right-padding (hdemucs.py:132-135) and lets the next layer's stride-4 window be
-            # a (pos/4, pos%4) TMA box.
-            Tin, Tout = tl[i], tl[i + 1]
-            y = self._buf(key, "y_t", B * Tout * Cc)
-            first = i == 0
-            Tin_p = Tin if first else tp(Tin)
-            conv0 = first and self.mode != "fp32" and Cc == 48 and A == 2     # dedicated mma.sync first-layer kernel
-            if conv0:
-                self._k("bd_encoder_conv0", ptr(xt), 1, norm.data_ptr() + 16, 8, ptr(W[f"tencoder.{i}.conv.w"]),
-                        ptr(W[f"tencoder.{i}.conv.b"]), ptr(y), B, 1, Tout, L, A, Cc, self.thin_math, self._stream(),
-                        flops=2.0 * B * Tout * Cc * 8 * A, nbytes=4.0 * B * (A * L + Tout * Cc), label="encoder_conv0_mma",
-                        detail=f"M={B * Tout} cin={A}")
-            else:
-              self._gemm(M=B * Tout, N=Cc, Cin=Cin_t, x=xt, w=W[f"tencoder.{i}.conv.w"], bias=W[f"tencoder.{i}.conv.b"],
-                       out=y, taps=tuple((0, k - 2) for k in range(8)), I1=1, I0=Tout, m0=4, J1=1, J0=Tin_p,
-                       xs=(A * L, 0, 1, L) if first else (Tin_p * Cin_t, 0, Cin_t, 1), os_=(Tout * Cc, 0, Cc),
-                       a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE,
-                       a_stats=norm[4:] if first else None, a_stats_stride=8, act=_lib.ACT_GELU)
-            if cfg.dconv_mode & 1:
-                self._dconv(key, f"tencoder.{i}", y, B, Tout, 1, Cc, "_t")
-            z = self._buf(key, f"saved_t{i}", B * tp(Tout) * Cc, zero=True)
-            self._gemm(M=B * Tout, N=2 * Cc, Cin=Cc, x=y, w=W[f"tencoder.{i}.rewrite.w"],
-                       bias=W[f"tencoder.{i}.rewrite.b"], out=z, act=_lib.ACT_GLU, I1=1, I0=Tout, J1=1, J0=Tout,
-                       xs=(Tout * Cc, 0, Cc, 1), os_=(tp(Tout) * Cc, 0, Cc))
-            saved_t.append(z)
-            xt, Cin_t = z, Cc
-            tap(f"tenc{i}", z.view(B, tp(Tout), Cc)[:, :Tout], "t")
-
-            # frequency branch: Conv2d(k=(8,1),s=(4,1),p=(2,0)) -> GELU
-            Fo = Fin // 4
-            y = self._buf(key, "y_f", B * T * Fo * Cc)
-            if conv0 and Cin == 4:
-                self._k("bd_encoder_conv0", ptr(xf), 0, ptr(norm), 8, ptr(W[f"encoder.{i}.conv.w"]),
-                        ptr(W[f"encoder.{i}.conv.b"]), ptr(y), B, T, Fo, Fin, Cin, Cc, self.thin_math, self._stream(),
-                        flops=2.0 * B * T * Fo * Cc * 8 * Cin, nbytes=4.0 * B * T * (Fin * Cin + Fo * Cc),
-                        label="encoder_conv0_mma", detail=f"M={B * T * Fo} cin={Cin}")
-            else:
-              self._gemm(M=B * T * Fo, N=Cc, Cin=Cin, x=xf, w=W[f"encoder.{i}.conv.w"], bias=W[f"encoder.{i}.conv.b"],
-                       out=y, taps=tuple((0, k - 2) for k in range(8)), I1=T, I0=Fo, m0=4, J1=T, J0=Fin,
-                       xs=(T * Fin * Cin, Fin * Cin, Cin, 1), os_=(T * Fo * Cc, Fo * Cc, Cc),
-                       a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE,
-                       a_stats=norm if first else None, a_stats_stride=8, act=_lib.ACT_GELU)
-            if cfg.dconv_mode & 1:
-                self._dconv(key, f"encoder.{i}", y, B, T, Fo, Cc, "_f")
-            z = self._buf(key, f"saved_f{i}", B * T * Fo * Cc)
-            emb = W["freq_emb"] if (first and cfg.freq_emb) else None
-            self._gemm(M=B * T * Fo, N=2 * Cc, Cin=Cc, x=y, w=W[f"encoder.{i}.rewrite.w"],
-                       bias=W[f"encoder.{i}.rewrite.b"], out=z, act=_lib.ACT_GLU,
-                       rowbias=emb, rowbias_period=Fo if emb is not None else 0)
-            saved.append(z)
-            xf, Fin, Cin = z, Fo, Cc
-            tap(f"enc{i}", z.view(B, T, Fo, Cc), "f")
+            xt = self._time_encoder(key, i, xt, "y_t", norm, taps, B, tl[i], tl[i + 1], Cin_t, Cc)
+            xf = self._freq_encoder(key, i, xf, "y_f", norm, taps, B, T, Fin, Cin, Cc)
+            saved_t.append(xt)
+            saved.append(xf)
+            Fin, Cin, Cin_t = Fin // 4, Cc, Cc
 
         Fb, Cb, T2 = Fin, chans[-1], tl[-1]
         Mf, Mt = B * T * Fb, B * T2
         # ping-pong buffers of the decoders, sized for their largest activation
         dec_f_numel = B * T * max(2048 * 4 * S, 512 * chans[0])
-        dec_t_numel = B * max(tp(L) * 2 * S, tp(tl[1]) * chans[0])
+        dec_t_numel = B * max(_pitch(L) * 2 * S, _pitch(tl[1]) * chans[0])
+
+        xd = self._buf(key, "dec_a", dec_f_numel)[: Mf * Cb]
+        xtd = self._buf(key, "dec_ta", dec_t_numel)[: B * _pitch(T2) * Cb]
 
         # ---- cross-domain transformer ------------------------------------------------------------
         if cfg.t_layers > 0:
             D = cfg.transformer_dim
+            x = self._buf(key, "tr_x", Mf * D)
+            xt_ = self._buf(key, "tr_xt", Mt * D)
             if cfg.bottom_channels:
-                x = self._buf(key, "tr_x", Mf * D)
-                xt_ = self._buf(key, "tr_xt", Mt * D)
                 self._gemm(M=Mf, N=D, Cin=Cb, x=xf, w=W["channel_upsampler.w"], bias=W["channel_upsampler.b"], out=x)
                 self._gemm(M=Mt, N=D, Cin=Cb, x=xt, w=W["channel_upsampler_t.w"], bias=W["channel_upsampler_t.b"],
-                           out=xt_, I1=1, I0=T2, J1=1, J0=T2, xs=(tp(T2) * Cb, 0, Cb, 1), os_=(T2 * D, 0, D))
+                           out=xt_, I1=1, I0=T2, J1=1, J0=T2, xs=(_pitch(T2) * Cb, 0, Cb, 1), os_=(T2 * D, 0, D))
             else:
-                x = self._buf(key, "tr_x", Mf * D)
-                xt_ = self._buf(key, "tr_xt", Mt * D)
                 x.copy_(xf)
-                xt_.view(B, T2, D).copy_(xt.view(B, tp(T2), Cb)[:, :T2])
+                xt_.view(B, T2, D).copy_(xt.view(B, _pitch(T2), Cb)[:, :T2])
             ct = "crosstransformer"
             pos2d = self._pos_table(("2d", Fb, T))
             pos1d = self._pos_table(("1d", T2))
@@ -662,32 +740,27 @@ class Engine:
                     self._ln(x, kt, f"{ct}.layers_t.{i}.norm2", Mf)
                     self._transformer_layer(key, x, kf, f"{ct}.layers.{i}", True, B, T * Fb, T2, "_f")
                     self._transformer_layer(key, xt_, kt, f"{ct}.layers_t.{i}", True, B, T2, T * Fb, "_t")
-                tap(f"xf.layer{i}", x.view(B, T, Fb, D), "f")
-                tap(f"xt.layer{i}", xt_.view(B, T2, D), "t")
+                _tap(taps, f"xf.layer{i}", x.view(B, T, Fb, D), "f")
+                _tap(taps, f"xt.layer{i}", xt_.view(B, T2, D), "t")
             # channel_downsampler (+ the decoder's skip add, hdemucs.py:310, fused as `addend`)
-            xd = self._buf(key, "dec_a", dec_f_numel)[: Mf * Cb]
-            xtd = self._buf(key, "dec_ta", dec_t_numel)[: B * tp(T2) * Cb]
             if cfg.bottom_channels:
                 self._gemm(M=Mf, N=Cb, Cin=D, x=x, w=W["channel_downsampler.w"], bias=W["channel_downsampler.b"],
                            out=xd, addend=saved[-1])
                 self._gemm(M=Mt, N=Cb, Cin=D, x=xt_, w=W["channel_downsampler_t.w"],
                            bias=W["channel_downsampler_t.b"], out=xtd, addend=saved_t[-1], I1=1, I0=T2, J1=1, J0=T2,
-                           xs=(T2 * D, 0, D, 1), os_=(tp(T2) * Cb, 0, Cb))
+                           xs=(T2 * D, 0, D, 1), os_=(_pitch(T2) * Cb, 0, Cb))
             else:
                 torch.add(x, saved[-1], out=xd)
-                xtd.view(B, tp(T2), Cb)[:, :T2].copy_(xt_.view(B, T2, Cb) + saved_t[-1].view(B, tp(T2), Cb)[:, :T2])
+                xtd.view(B, _pitch(T2), Cb)[:, :T2].copy_(xt_.view(B, T2, Cb) + saved_t[-1].view(B, _pitch(T2), Cb)[:, :T2])
             if taps is not None:
-                tap("bottleneck", (xd - saved[-1]).view(B, T, Fb, Cb), "f")
-                tap("bottleneck_t", (xtd - saved_t[-1]).view(B, tp(T2), Cb)[:, :T2], "t")
+                _tap(taps, "bottleneck", (xd - saved[-1]).view(B, T, Fb, Cb), "f")
+                _tap(taps, "bottleneck_t", (xtd - saved_t[-1]).view(B, _pitch(T2), Cb)[:, :T2], "t")
         else:
-            xd = self._buf(key, "dec_a", dec_f_numel)[: Mf * Cb]
-            xtd = self._buf(key, "dec_ta", dec_t_numel)[: B * tp(T2) * Cb]
             torch.add(xf, saved[-1], out=xd)
             torch.mul(saved_t[-1], 2.0, out=xtd)    # no transformer: x + skip with skip == x
 
         # ---- decoders ------------------------------------------------------------------------------
         Fcur = Fb
-        names = ("dec_a", "dec_b")
         for j in range(cfg.depth):
             Cc = chans[cfg.depth - 1 - j]
             last = j == cfg.depth - 1
@@ -695,53 +768,12 @@ class Engine:
             Cout_t = 2 * S if last else Cc // 2
             skip = None if last else saved[cfg.depth - 2 - j]
             skip_t = None if last else saved_t[cfg.depth - 2 - j]
-            # frequency: 3x3 rewrite + GLU (hdemucs.py:312-313)
-            y = self._buf(key, "y_f", B * T * Fcur * Cc)
-            taps9 = tuple((kt - 1, kf - 1) for kf in range(3) for kt in range(3))
-            self._gemm(M=B * T * Fcur, N=2 * Cc, Cin=Cc, x=xd, w=W[f"decoder.{j}.rewrite.w"],
-                       bias=W[f"decoder.{j}.rewrite.b"], out=y, taps=taps9, I1=T, I0=Fcur, J1=T, J0=Fcur,
-                       xs=(T * Fcur * Cc, Fcur * Cc, Cc, 1), os_=(T * Fcur * Cc, Fcur * Cc, Cc), act=_lib.ACT_GLU)
-            if cfg.dconv_mode & 2:
-                self._dconv(key, f"decoder.{j}", y, B, T, Fcur, Cc, "_f")
-            # ConvTranspose2d(k=(8,1), s=(4,1)) + crop [2:-2] + GELU (+ next skip) (hdemucs.py:326-334)
-            nxt = self._buf(key, names[(j + 1) % 2], dec_f_numel)[: B * T * 4 * Fcur * Cout]
-            three = self.mode != "fp32" and 4 * Cout >= 64   # tensor-core form: no halo row
-            self._gemm(M=B * T * (Fcur + (0 if three else 1)), N=4 * Cout, Cin=Cc, x=y,
-                       w=W[f"decoder.{j}.conv_tr.w3" if three else f"decoder.{j}.conv_tr.w"],
-                       bias=W[f"decoder.{j}.conv_tr.b"], out=nxt,
-                       taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=T,
-                       I0=Fcur + (0 if three else 1), J1=T, J0=Fcur, xs=(T * Fcur * Cc, Fcur * Cc, Cc, 1),
-                       # the last layer writes source-major [B, T, S, F, 4] so that an iSTFT frame is contiguous
-                       os_=(T * 4 * Fcur * Cout, 4 * Fcur * Cout, 4 if last else Cout),
-                       oc_split=4 if last else 0, oc_stride=4 * Fcur * 4 if last else 0,
-                       convt=2 if three else 1, O0=4 * Fcur,
-                       act=_lib.ACT_NONE if last else _lib.ACT_GELU, addend=skip)
-            if taps is not None:
-                if last:   # [B,T,S,F,4] -> [B,T,F,(s j)]
-                    tap(f"dec{j}", nxt.view(B, T, S, 4 * Fcur, 4).permute(0, 1, 3, 2, 4).reshape(B, T, 4 * Fcur, Cout), "f")
-                else:
-                    tap(f"dec{j}", (nxt - skip).view(B, T, 4 * Fcur, Cout), "f")
+            nxt = self._buf(key, ("dec_a", "dec_b")[(j + 1) % 2], dec_f_numel)[: B * T * 4 * Fcur * Cout]
+            self._freq_decoder(key, j, xd, "y_f", nxt, skip, taps, B, T, Fcur, Cc, Cout)
             xd, Fcur = nxt, 4 * Fcur
-
-            # time: k=3 rewrite + GLU, DConv, ConvTranspose1d(k=8,s=4) + crop [2:2+length] + GELU
             Tin, Tout = tl[cfg.depth - j], tl[cfg.depth - 1 - j]
-            y = self._buf(key, "y_t", B * Tin * Cc)
-            self._gemm(M=B * Tin, N=2 * Cc, Cin=Cc, x=xtd, w=W[f"tdecoder.{j}.rewrite.w"],
-                       bias=W[f"tdecoder.{j}.rewrite.b"], out=y, taps=((0, -1), (0, 0), (0, 1)), I1=1, I0=Tin,
-                       J1=1, J0=Tin, xs=(tp(Tin) * Cc, 0, Cc, 1), os_=(Tin * Cc, 0, Cc), act=_lib.ACT_GLU)
-            if cfg.dconv_mode & 2:
-                self._dconv(key, f"tdecoder.{j}", y, B, Tin, 1, Cc, "_t")
-            nxt = self._buf(key, "dec_tb" if (j % 2 == 0) else "dec_ta", dec_t_numel)[: B * tp(Tout) * Cout_t]
-            three = self.mode != "fp32" and 4 * Cout_t >= 64
-            self._gemm(M=B * (Tin + (0 if three else 1)), N=4 * Cout_t, Cin=Cc, x=y,
-                       w=W[f"tdecoder.{j}.conv_tr.w3" if three else f"tdecoder.{j}.conv_tr.w"],
-                       bias=W[f"tdecoder.{j}.conv_tr.b"], out=nxt,
-                       taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=1,
-                       I0=Tin + (0 if three else 1), J1=1, J0=Tin, xs=(Tin * Cc, 0, Cc, 1),
-                       os_=(tp(Tout) * Cout_t, 0, Cout_t), convt=2 if three else 1, O0=Tout,
-                       act=_lib.ACT_NONE if last else _lib.ACT_GELU, addend=skip_t)
-            if taps is not None:
-                tap(f"tdec{j}", (nxt - skip_t if skip_t is not None else nxt).view(B, tp(Tout), Cout_t)[:, :Tout], "t")
+            nxt = self._buf(key, ("dec_ta", "dec_tb")[(j + 1) % 2], dec_t_numel)[: B * _pitch(Tout) * Cout_t]
+            self._time_decoder(key, j, xtd, "y_t", nxt, skip_t, taps, B, Tin, Tout, Cc, Cout_t)
             xtd = nxt
 
         if mag is not None:
@@ -749,24 +781,14 @@ class Engine:
             nm = norm.view(B, 8)
             spec_out = xd[: B * T * S * 2048 * 2 * A].view(B, T, S, 2048, 2 * A).permute(0, 2, 4, 3, 1)
             spec_out = spec_out * nm[:, 1].view(B, 1, 1, 1, 1) + nm[:, 0].view(B, 1, 1, 1, 1)
-            time_out = xtd[: B * tp(L) * A * S].view(B, tp(L), S, A)[:, :L].permute(0, 2, 3, 1)
+            time_out = xtd[: B * _pitch(L) * A * S].view(B, _pitch(L), S, A)[:, :L].permute(0, 2, 3, 1)
             time_out = time_out * nm[:, 5].view(B, 1, 1, 1) + nm[:, 4].view(B, 1, 1, 1)
             return spec_out.contiguous(), time_out.contiguous()
-        # ---- K2: de-normalise, iSTFT, overlap-add in shared memory, crop, add the time branch ------------
-        if out_buf is not None:
-            if out_buf.numel() != B * S * A * L0 or out_buf.dtype != torch.float32 or out_buf.device != self.device \
-                    or not out_buf.is_contiguous():
-                raise ValueError("out must be a contiguous float32 tensor of B*S*C*L elements on the engine's device")
-            out = out_buf.view(B, S, A, L0)
-        else:
-            out = torch.empty(B, S, A, L0, dtype=torch.float32, device=self.device)
-        self._k("bd_istft_ola", ptr(xd), ptr(norm), ptr(self.window), ptr(self.twiddle), ptr(xtd), ptr(out),
-                B, S, T, tp(L), L0, st, nbytes=4.0 * B * S * (T * 2048 * 4 + 2 * L + 2 * L0),
-                flops=2.5 * 4096 * 12 * 2 * S * B * T)
+        out = self._istft(xd, xtd, norm, out_buf, B, T, L, L0)
         if taps is not None:
             only = torch.empty(B, S, A, L0, dtype=torch.float32, device=self.device)
             self._k("bd_istft_ola", ptr(xd), ptr(norm), ptr(self.window), ptr(self.twiddle), None, ptr(only),
-                    B, S, T, tp(L), L0, st)
+                    B, S, T, _pitch(L), L0, self._stream())
             taps["istft"] = only
             taps["time_out"] = out - only
         return out

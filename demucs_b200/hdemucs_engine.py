@@ -1,8 +1,8 @@
 """Host-side orchestration of the Hybrid Demucs v3 forward on the sm_100a kernel library.
 
 Python mirror of ``HDemucs.forward`` (reference demucs/hdemucs.py:689-794) for the hdemucs_mmi family, as a sequence of
-C-ABI launches.  It shares the plumbing, the spectral kernels and the implicit-GEMM convolutions with the HTDemucs
-``Engine``; what is specific to v3:
+C-ABI launches.  It is an HTDemucs ``Engine`` with another weight packing: the STFT / iSTFT and the HTDemucs-style
+encoder / decoder layers are the ``Engine``'s own steps; what is specific to v3:
 
 * layers 0-3 are the HTDemucs encoder / decoder layers without a decoder DConv (``dconv_mode=1``) and with
   ``dconv_comp=4`` (hidden widths 12 / 24 / 48 / 96);
@@ -23,12 +23,11 @@ from __future__ import annotations
 import math
 import typing as tp
 
-import numpy as np
 import torch
 
 from . import _lib
 from ._lib import ptr
-from .engine import Engine, MODES, conv_w, convtr_w, convtr_w3, pack_dconv, _interleave_glu
+from .engine import Engine, _conv3_geometry, _pitch, _tap, conv_w, convtr_w, pack_dconv, pack_decoder, pack_encoder
 from .hdemucs import HDemucsConfig, param_specs
 
 
@@ -63,10 +62,12 @@ class HDemucsWeights:
             # DConv: (conv3, norm1, [BLSTM], [LocalState], conv1x1, norm2, GLU, LayerScale) -- demucs.py:133-150
             k = 3 + int(l["lstm"]) + int(l["attn"])
             idx = (0, 1, k, k + 1, k + 3)
-            put(f"{e}.conv.b", f32(f"{e}.conv.bias"))
             put(f"{e}.rewrite.b_nat", f32(f"{e}.rewrite.bias"))
-            if l["norm"]:
+            if not l["norm"]:
+                pack_encoder(put, state, e)
+            else:
                 # GroupNorm'd layers keep the reference's channel order: the GLU runs after the norm, in bd_gn_act
+                put(f"{e}.conv.b", f32(f"{e}.conv.bias"))
                 put(f"{e}.rewrite.w", conv_w(f32(f"{e}.rewrite.weight")))
                 put(f"{e}.rewrite.b", f32(f"{e}.rewrite.bias"))
                 for n in ("norm1", "norm2"):
@@ -74,20 +75,15 @@ class HDemucsWeights:
                     put(f"{e}.{n}.b", f32(f"{e}.{n}.bias"))
                     put(f"{d}.{n}.g", f32(f"{d}.{n}.weight"))
                     put(f"{d}.{n}.b", f32(f"{d}.{n}.bias"))
-            else:
-                put(f"{e}.rewrite.w", _interleave_glu(conv_w(f32(f"{e}.rewrite.weight"))))
-                put(f"{e}.rewrite.b", _interleave_glu(f32(f"{e}.rewrite.bias")))
-            if l["freq"] and not l["last_freq"]:
-                put(f"{e}.conv.w", conv_w(f32(f"{e}.conv.weight")))
-            elif l["last_freq"]:
-                put(f"{e}.conv.w", conv_w(f32(f"{e}.conv.weight")))                       # [Cout, 8*Cin]: one dense row per frame
-            else:
-                # Conv1d(k=4, s=2, p=1) over position PAIRS: out[t] = w0 x[2t-1] + w1 x[2t] + w2 x[2t+1] + w3 x[2t+2];
-                # pair rows [x[2p] | x[2p+1]], taps (-1, 0, +1) with zero blocks where a tap does not reach
-                w = f32(f"{e}.conv.weight")                                               # [Cout, Cin, 4]
-                co, ci = w.shape[:2]
-                z = w.new_zeros(co, ci)
-                put(f"{e}.conv.wpair", torch.cat([z, w[:, :, 0], w[:, :, 1], w[:, :, 2], w[:, :, 3], z], dim=1))
+                if l["last_freq"]:
+                    put(f"{e}.conv.w", conv_w(f32(f"{e}.conv.weight")))                   # [Cout, 8*Cin]: one dense row per frame
+                else:
+                    # Conv1d(k=4, s=2, p=1) over position PAIRS: out[t] = w0 x[2t-1] + w1 x[2t] + w2 x[2t+1] + w3 x[2t+2];
+                    # pair rows [x[2p] | x[2p+1]], taps (-1, 0, +1) with zero blocks where a tap does not reach
+                    w = f32(f"{e}.conv.weight")                                           # [Cout, Cin, 4]
+                    co, ci = w.shape[:2]
+                    z = w.new_zeros(co, ci)
+                    put(f"{e}.conv.wpair", torch.cat([z, w[:, :, 0], w[:, :, 1], w[:, :, 2], w[:, :, 3], z], dim=1))
             pack_dconv(put, self.t, state, e, cfg.dconv_depth, tc_forms, idx)
             if big:
                 hid = state[f"{e}.dconv.layers.0.0.weight"].shape[0]
@@ -128,30 +124,21 @@ class HDemucsWeights:
                     put(f"{d}.conv_tr.w", w.reshape(ci, co, 2, 2).permute(3, 1, 2, 0).reshape(2 * co, 2 * ci))
                     put(f"{d}.conv_tr.b", f32(f"{d}.conv_tr.bias").repeat(2))
             else:
-                put(f"{d}.rewrite.w", _interleave_glu(conv_w(f32(f"{d}.rewrite.weight"))))
-                put(f"{d}.rewrite.b", _interleave_glu(f32(f"{d}.rewrite.bias")))
-                put(f"{d}.conv_tr.w", convtr_w(f32(f"{d}.conv_tr.weight")))
-                if tc_forms:
-                    put(f"{d}.conv_tr.w3", convtr_w3(f32(f"{d}.conv_tr.weight")))
-                put(f"{d}.conv_tr.b", f32(f"{d}.conv_tr.bias").repeat(4))
+                pack_decoder(put, state, d, tc_forms)
             if not l["has_time"]:
                 continue
             te, td = f"tencoder.{i}", f"tdecoder.{n_time - 1 - i}"
-            put(f"{te}.conv.w", conv_w(f32(f"{te}.conv.weight")))
-            put(f"{te}.conv.b", f32(f"{te}.conv.bias"))
-            put(f"{td}.conv_tr.w", convtr_w(f32(f"{td}.conv_tr.weight")))
-            put(f"{td}.conv_tr.b", f32(f"{td}.conv_tr.bias").repeat(4))
-            if l["time_empty"]:
+            if l["time_empty"]:    # conv-only layers (hdemucs.py:137-143); the decoder's GroupNorm runs before its crop
+                put(f"{te}.conv.w", conv_w(f32(f"{te}.conv.weight")))
+                put(f"{te}.conv.b", f32(f"{te}.conv.bias"))
+                put(f"{td}.conv_tr.w", convtr_w(f32(f"{td}.conv_tr.weight")))
+                put(f"{td}.conv_tr.b", f32(f"{td}.conv_tr.bias").repeat(4))
                 put(f"{td}.norm2.g", f32(f"{td}.norm2.weight"))
                 put(f"{td}.norm2.b", f32(f"{td}.norm2.bias"))
                 continue
-            if tc_forms:
-                put(f"{td}.conv_tr.w3", convtr_w3(f32(f"{td}.conv_tr.weight")))
-            put(f"{te}.rewrite.w", _interleave_glu(conv_w(f32(f"{te}.rewrite.weight"))))
-            put(f"{te}.rewrite.b", _interleave_glu(f32(f"{te}.rewrite.bias")))
+            pack_encoder(put, state, te)
             pack_dconv(put, self.t, state, te, cfg.dconv_depth, tc_forms)
-            put(f"{td}.rewrite.w", _interleave_glu(conv_w(f32(f"{td}.rewrite.weight"))))
-            put(f"{td}.rewrite.b", _interleave_glu(f32(f"{td}.rewrite.bias")))
+            pack_decoder(put, state, td, tc_forms)
         if cfg.freq_emb:
             put("freq_emb", cfg.freq_emb * cfg.emb_scale * f32("freq_emb.embedding.weight"))
 
@@ -162,29 +149,10 @@ class HDemucsWeights:
 class HDemucsEngine(Engine):
     """One HDemucs (v3) model resident on one GPU."""
 
+    Weights = HDemucsWeights
+
     def __init__(self, cfg: HDemucsConfig, state, device="cuda", mode: str = "strict"):
-        cfg.validate()
-        if mode not in MODES:
-            raise ValueError(f"mode must be one of {MODES}")
-        self.cfg = cfg
-        self.mode = mode
-        self.device = torch.device(device)
-        if self.device.type != "cuda" and _lib.TEST_HOOK is None:
-            raise _lib.KernelError("demucs_b200 runs on CUDA devices only (there is no CPU path)")
-        _lib.lib()
-        self.W = HDemucsWeights(cfg, state, self.device, tc_forms=(mode != "fp32"))
-        k = np.arange(cfg.nfft, dtype=np.float64)
-        self.window = torch.from_numpy((0.5 - 0.5 * np.cos(2 * np.pi * k / cfg.nfft)).astype(np.float32)).to(self.device)
-        tw = np.stack([np.cos(2 * np.pi * k / cfg.nfft), -np.sin(2 * np.pi * k / cfg.nfft)], axis=1)
-        self.twiddle = torch.from_numpy(tw.astype(np.float32)).to(self.device).contiguous()
-        self.single_pass = mode in ("tf32", "bf16")
-        self.thin_math = {"tf32": _lib.MATH_TF32, "bf16": _lib.MATH_BF16, "tf32x3": _lib.MATH_TF32X3,
-                          "strict": _lib.MATH_BF16X3}.get(mode)
-        self._w16_cache = {}
-        self._bufs = {}
-        self._pos = {}
-        self.launches = 0
-        self._prof = None
+        super().__init__(cfg, state, device, mode)
 
     # ------------------------------------------------------------------ GroupNorm(4) helpers
     def _gn(self, key, x, y, p: str, B: int, rows_in: int, C_: int, act: int, row0: int = 0, rows_out: tp.Optional[int] = None,
@@ -221,13 +189,8 @@ class HDemucsEngine(Engine):
         for dd in range(cfg.dconv_depth):
             p = f"{prefix}.dconv.layers.{dd}"
             dil = 2 ** dd
-            if Fr == 1:
-                geo = dict(taps=((0, -dil), (0, 0), (0, dil)), I1=1, I0=T, J1=1, J0=T, xs=(T * C_, 0, C_, 1), os_=(T * hp, 0, hp))
-            else:
-                geo = dict(taps=((-dil, 0), (0, 0), (dil, 0)), I1=T, I0=Fr, J1=T, J0=Fr,
-                           xs=(T * Fr * C_, Fr * C_, C_, 1), os_=(T * Fr * hp, Fr * hp, hp))
             self._gemm(M=M, N=hp, Cin=C_, x=x, w=W[f"{p}.w1{sfx}"], bias=W[f"{p}.b1{sfx}"], out=h, stats_out=sums, stat=stat,
-                       tc=tc, **geo)
+                       tc=tc, **_conv3_geometry(T, Fr, C_, hp, dil))
             self._k("bd_finalize_group_stats", ptr(sums), ptr(mr1), slabs, float(T * hid), st)
             self._k("bd_gn_gelu_apply", ptr(h), ptr(mr1), ptr(W[f"{p}.g1{sfx}"]), ptr(W[f"{p}.be1{sfx}"]), M, hp, T * Fr, Fr, st,
                     nbytes=8.0 * M * hp, label="bd_gn_gelu_apply")
@@ -288,51 +251,28 @@ class HDemucsEngine(Engine):
                 nbytes=4.0 * B * T * 4 * D, label="local_state")
         self._gemm(M=B * T, N=D, Cin=D, x=res, w=W[f"{p}.attn.proj.w"], bias=W[f"{p}.attn.proj.b"], out=h, resid=h)
 
-    def _dconv_any(self, key, prefix, x, B, T, Fr, C_, l: dict, tag: str):
-        hid = int(C_ / self.cfg.dconv_comp)
-        if l["lstm"] or l["attn"] or hid > 48:
-            self._dconv_big(key, prefix, x, B, T, Fr, C_, l["lstm"], l["attn"], tag)
+    def _dconv(self, key, prefix, x, B, T, Fr, C_, tag: str, lstm: bool = False, attn: bool = False):
+        """DConv of a v3 layer: with BLSTM / LocalState or a hidden width beyond the register kernels (> 48) it is
+        ``_dconv_big``, otherwise the HTDemucs form."""
+        if lstm or attn or int(C_ / self.cfg.dconv_comp) > 48:
+            self._dconv_big(key, prefix, x, B, T, Fr, C_, lstm, attn, tag)
         else:
-            self._dconv(key, prefix, x, B, T, Fr, C_, tag)
+            super()._dconv(key, prefix, x, B, T, Fr, C_, tag)
 
     # ------------------------------------------------------------------ forward
     def forward_core(self, mag, mix):
         raise NotImplementedError("forward_core is the HTDemucs ONNX surface (htdemucs.py:662-759)")
 
-    def _forward(self, mix: torch.Tensor, taps: tp.Optional[dict], out_buf: tp.Optional[torch.Tensor], mag=None):
+    def _forward(self, mix: torch.Tensor, taps: tp.Optional[dict], out_buf: tp.Optional[torch.Tensor]):
         cfg, W = self.cfg, self.W
-        if mix.dim() != 3 or mix.shape[1] != cfg.audio_channels:
-            raise ValueError(f"expected mix of shape [B, {cfg.audio_channels}, L], got {tuple(mix.shape)}")
-        if mix.device != self.device or mix.dtype != torch.float32:
-            raise ValueError("mix must be a float32 tensor on the engine's device")
         B, A, L = mix.shape
         if L < 2560:     # the reflect padding of _spec (1536 + up to 1023 samples) must stay inside the signal; the
             raise ValueError("input shorter than 2560 samples: the small-input guard of pad1d (hdemucs.py:29-36) is not built")
         mix = mix.contiguous()
         key = (B, L)
-        st = self._stream()
-        S = cfg.n_sources
         T = cfg.frames(L)
         layers = cfg.layers()
-        tc = self.mode != "fp32"
-
-        def tp4(n):
-            return (n + 3) // 4 * 4
-
-        def tap(name, t, fmt):
-            if taps is None:
-                return
-            taps[name] = (t.permute(0, 3, 2, 1) if fmt == "f" else t.permute(0, 2, 1)).clone()
-
-        # ---- K1: STFT + CaC pack + normalisation statistics (hdemucs.py:693-709) ----------------------------
-        spec = self._buf(key, "spec", B * T * 2048 * 4)
-        stats = self._buf(key, "item_stats", 4 * B, torch.float64)
-        norm = self._buf(key, "item_norm", 8 * B)
-        stats.zero_()
-        self._k("bd_stft_cac", ptr(mix), ptr(self.window), ptr(self.twiddle), ptr(spec), ptr(stats), B, A, L, st,
-                nbytes=4.0 * B * (A * L + T * 2048 * 4), flops=2.5 * 4096 * 12 * 2 * B * T)
-        self._k("bd_finalize_item_norm", ptr(stats), ptr(norm), B, float(4 * 2048 * T), float(A * L), st)
-        tap("stft", spec.view(B, T, 2048, 4), "f")
+        spec, norm = self._stft(key, mix, taps)        # hdemucs.py:693-709
 
         # ---- encoders --------------------------------------------------------------------------------------------
         tl = [L]
@@ -348,56 +288,17 @@ class HDemucsEngine(Engine):
         T5 = (T + 1) // 2        # Conv1d(k=4, s=2, p=1) after right-padding T to even
         for l in layers:
             i, Cc = l["index"], l["chout_z"]
-            first = i == 0
-            if l["has_time"]:
-                Tin, Tout = tl[i], tl[i + 1]
-                Tin_p = Tin if first else tp4(Tin)
-                y = self._buf(key, f"y_t{i}", B * Tout * Cc)
-                conv0 = first and tc and Cc == 48 and A == 2
-                if conv0:
-                    self._k("bd_encoder_conv0", ptr(xt), 1, norm.data_ptr() + 16, 8, ptr(W[f"tencoder.{i}.conv.w"]),
-                            ptr(W[f"tencoder.{i}.conv.b"]), ptr(y), B, 1, Tout, L, A, Cc, self.thin_math, st,
-                            flops=2.0 * B * Tout * Cc * 8 * A, nbytes=4.0 * B * (A * L + Tout * Cc), label="encoder_conv0_mma")
-                else:
-                    self._gemm(M=B * Tout, N=Cc, Cin=Cin_t, x=xt, w=W[f"tencoder.{i}.conv.w"], bias=W[f"tencoder.{i}.conv.b"],
-                               out=y, taps=tuple((0, k - 2) for k in range(8)), I1=1, I0=Tout, m0=4, J1=1, J0=Tin_p,
-                               xs=(A * L, 0, 1, L) if first else (Tin_p * Cin_t, 0, Cin_t, 1), os_=(Tout * Cc, 0, Cc),
-                               a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE, a_stats=norm[4:] if first else None,
-                               a_stats_stride=8, act=_lib.ACT_NONE if l["time_empty"] else _lib.ACT_GELU)
-                if l["time_empty"]:
-                    inject = y                         # conv only; added to the frequency branch below (hdemucs.py:137-143)
-                    tap(f"tenc{i}", y.view(B, Tout, Cc), "t")
-                else:
-                    self._dconv_any(key, f"tencoder.{i}", y, B, Tout, 1, Cc, l, "_t")
-                    z = self._buf(key, f"saved_t{i}", B * tp4(Tout) * Cc, zero=True)
-                    self._gemm(M=B * Tout, N=2 * Cc, Cin=Cc, x=y, w=W[f"tencoder.{i}.rewrite.w"],
-                               bias=W[f"tencoder.{i}.rewrite.b"], out=z, act=_lib.ACT_GLU, I1=1, I0=Tout, J1=1, J0=Tout,
-                               xs=(Tout * Cc, 0, Cc, 1), os_=(tp4(Tout) * Cc, 0, Cc))
-                    saved_t.append(z)
-                    xt, Cin_t = z, Cc
-                    tap(f"tenc{i}", z.view(B, tp4(Tout), Cc)[:, :Tout], "t")
+            if l["time_empty"]:     # conv only; added to the frequency branch below (hdemucs.py:137-143)
+                inject = self._time_encoder(key, i, xt, f"y_t{i}", norm, taps, B, tl[i], tl[i + 1], Cin_t, Cc, conv_only=True)
+            elif l["has_time"]:
+                xt = self._time_encoder(key, i, xt, f"y_t{i}", norm, taps, B, tl[i], tl[i + 1], Cin_t, Cc)
+                saved_t.append(xt)
+                Cin_t = Cc
             e = f"encoder.{i}"
             if l["freq"] and not l["last_freq"]:
-                Fo = Fin // 4
-                y = self._buf(key, f"y_f{i}", B * T * Fo * Cc)
-                if first and tc and Cc == 48 and Cin == 4:
-                    self._k("bd_encoder_conv0", ptr(xf), 0, ptr(norm), 8, ptr(W[f"{e}.conv.w"]), ptr(W[f"{e}.conv.b"]), ptr(y),
-                            B, T, Fo, Fin, Cin, Cc, self.thin_math, st, flops=2.0 * B * T * Fo * Cc * 8 * Cin,
-                            nbytes=4.0 * B * T * (Fin * Cin + Fo * Cc), label="encoder_conv0_mma")
-                else:
-                    self._gemm(M=B * T * Fo, N=Cc, Cin=Cin, x=xf, w=W[f"{e}.conv.w"], bias=W[f"{e}.conv.b"], out=y,
-                               taps=tuple((0, k - 2) for k in range(8)), I1=T, I0=Fo, m0=4, J1=T, J0=Fin,
-                               xs=(T * Fin * Cin, Fin * Cin, Cin, 1), os_=(T * Fo * Cc, Fo * Cc, Cc),
-                               a_mode=_lib.A_ITEM_AFFINE if first else _lib.A_NONE, a_stats=norm if first else None,
-                               a_stats_stride=8, act=_lib.ACT_GELU)
-                self._dconv_any(key, e, y, B, T, Fo, Cc, l, "_f")
-                z = self._buf(key, f"saved_f{i}", B * T * Fo * Cc)
-                emb = W["freq_emb"] if (first and cfg.freq_emb) else None
-                self._gemm(M=B * T * Fo, N=2 * Cc, Cin=Cc, x=y, w=W[f"{e}.rewrite.w"], bias=W[f"{e}.rewrite.b"], out=z,
-                           act=_lib.ACT_GLU, rowbias=emb, rowbias_period=Fo if emb is not None else 0)
-                saved.append(z)
-                xf, Fin, Cin = z, Fo, Cc
-                tap(f"enc{i}", z.view(B, T, Fo, Cc), "f")
+                xf = self._freq_encoder(key, i, xf, f"y_f{i}", norm, taps, B, T, Fin, Cin, Cc)
+                saved.append(xf)
+                Fin, Cin = Fin // 4, Cc
                 continue
             # GroupNorm'd layers on the merged branch: rows = time steps, one "frequency" left
             if l["last_freq"]:
@@ -417,14 +318,14 @@ class HDemucsEngine(Engine):
                            taps=((0, -1), (0, 0), (0, 1)), I1=1, I0=rows, J1=1, J0=Tp // 2,
                            xs=(Tp * Cin, 0, 2 * Cin, 1), os_=(rows * Cc, 0, Cc))
             self._gn(key, raw, raw, f"{e}.norm1", B, rows, Cc, _lib.ACT_GELU, tag=f"_e{i}a")
-            self._dconv_any(key, e, raw, B, rows, 1, Cc, l, f"_m{i}")
+            self._dconv(key, e, raw, B, rows, 1, Cc, f"_m{i}", l["lstm"], l["attn"])
             rw = self._buf(key, f"rw{i}", B * rows * 2 * Cc)
             self._gemm(M=B * rows, N=2 * Cc, Cin=Cc, x=raw, w=W[f"{e}.rewrite.w"], bias=W[f"{e}.rewrite.b"], out=rw)
             z = self._buf(key, f"saved_f{i}", B * rows * Cc)
             self._gn(key, rw, z, f"{e}.norm2", B, rows, 2 * Cc, _lib.ACT_GLU, tag=f"_e{i}b")
             saved.append(z)
             xf, Fin, Cin = z, 1, Cc
-            tap(f"enc{i}", z.view(B, rows, 1, Cc), "f")
+            _tap(taps, f"enc{i}", z.view(B, rows, 1, Cc), "f")
 
         # ---- decoders: x starts at zero, so layer 0 reads its skip tensor alone (hdemucs.py:742-749) ---------------
         n_time = len(tl) - 1
@@ -452,7 +353,7 @@ class HDemucsEngine(Engine):
                 nxt = self._buf(key, f"dx{j}", B * T * Cout)
                 self._gn(key, full, nxt, f"{d}.norm2", B, 2 * rows + 2, Cout, _lib.ACT_GELU, row0=1, rows_out=T,
                          addend=nxt_skip, tag=f"_d{j}b")
-                tap(f"dec{j}", (nxt - nxt_skip).view(B, T, Cout), "t")
+                _tap(taps, f"dec{j}", (nxt - nxt_skip).view(B, T, Cout), "t")
                 xd = nxt
                 continue
             if l["norm"]:
@@ -467,7 +368,7 @@ class HDemucsEngine(Engine):
                 self._gemm(M=B * T, N=8 * Cout, Cin=Cc, x=pre, w=W[f"{d}.conv_tr.w"], bias=W[f"{d}.conv_tr.b"], out=full)
                 nxt = self._buf(key, f"dx{j}", B * T * 8 * Cout)
                 self._gn(key, full, nxt, f"{d}.norm2", B, T * 8, Cout, _lib.ACT_GELU, addend=nxt_skip, tag=f"_d{j}b")
-                tap(f"dec{j}", (nxt - nxt_skip).view(B, T, 8, Cout), "f")
+                _tap(taps, f"dec{j}", (nxt - nxt_skip).view(B, T, 8, Cout), "f")
                 xd, Fcur = nxt, 8
                 # time branch leaves the merged one here: conv_tr of `pre` only (empty layer), GroupNorm, crop, GELU
                 td = f"tdecoder.{j - (cfg.depth - n_time)}"
@@ -476,62 +377,23 @@ class HDemucsEngine(Engine):
                 self._gemm(M=B * (T + 1), N=4 * Ct, Cin=Cc, x=pre, w=W[f"{td}.conv_tr.w"], bias=W[f"{td}.conv_tr.b"], out=fullt,
                            taps=((0, 0), (0, -1)), I1=1, I0=T + 1, J1=1, J0=T, xs=(T * Cc, 0, Cc, 1),
                            os_=((T + 1) * 4 * Ct, 0, 4 * Ct))
-                xtd = self._buf(key, "tdx0", B * tp4(Tt) * Ct, zero=True)
+                xtd = self._buf(key, "tdx0", B * _pitch(Tt) * Ct, zero=True)
                 skip_t = saved_t[n_time - 2]
                 self._gn(key, fullt, xtd, f"{td}.norm2", B, 4 * T + 4, Ct, _lib.ACT_GELU, row0=2, rows_out=Tt, addend=skip_t,
-                         y_item_stride=tp4(Tt) * Ct, tag="_td0")
-                tap("tdec0", (xtd - skip_t).view(B, tp4(Tt), Ct)[:, :Tt], "t")
+                         y_item_stride=_pitch(Tt) * Ct, tag="_td0")
+                _tap(taps, "tdec0", (xtd - skip_t).view(B, _pitch(Tt), Ct)[:, :Tt], "t")
                 continue
             # ---- index 3..0: the HTDemucs decoder layers without DConv ------------------------------------------------
-            y = self._buf(key, f"dy{j}", B * T * Fcur * Cc)
-            taps9 = tuple((kt - 1, kf - 1) for kf in range(3) for kt in range(3))
-            self._gemm(M=B * T * Fcur, N=2 * Cc, Cin=Cc, x=xd, w=W[f"{d}.rewrite.w"], bias=W[f"{d}.rewrite.b"], out=y, taps=taps9,
-                       I1=T, I0=Fcur, J1=T, J0=Fcur, xs=(T * Fcur * Cc, Fcur * Cc, Cc, 1), os_=(T * Fcur * Cc, Fcur * Cc, Cc),
-                       act=_lib.ACT_GLU)
             nxt = self._buf(key, f"dx{j}", B * T * 4 * Fcur * Cout)
-            three = tc and 4 * Cout >= 64
-            self._gemm(M=B * T * (Fcur + (0 if three else 1)), N=4 * Cout, Cin=Cc, x=y,
-                       w=W[f"{d}.conv_tr.w3" if three else f"{d}.conv_tr.w"], bias=W[f"{d}.conv_tr.b"], out=nxt,
-                       taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=T,
-                       I0=Fcur + (0 if three else 1), J1=T, J0=Fcur, xs=(T * Fcur * Cc, Fcur * Cc, Cc, 1),
-                       os_=(T * 4 * Fcur * Cout, 4 * Fcur * Cout, 4 if last else Cout),
-                       oc_split=4 if last else 0, oc_stride=4 * Fcur * 4 if last else 0,
-                       convt=2 if three else 1, O0=4 * Fcur, act=_lib.ACT_NONE if last else _lib.ACT_GELU, addend=nxt_skip)
-            if taps is not None:
-                if last:
-                    tap(f"dec{j}", nxt.view(B, T, S, 4 * Fcur, 4).permute(0, 1, 3, 2, 4).reshape(B, T, 4 * Fcur, Cout), "f")
-                else:
-                    tap(f"dec{j}", (nxt - nxt_skip).view(B, T, 4 * Fcur, Cout), "f")
+            self._freq_decoder(key, j, xd, f"dy{j}", nxt, nxt_skip, taps, B, T, Fcur, Cc, Cout)
             xd, Fcur = nxt, 4 * Fcur
             jt = j - (cfg.depth - n_time)                      # 1..4
-            td = f"tdecoder.{jt}"
             Ct_in, Ct = l["chout"], l["dec_out"]
             Tin, Tout = tl[n_time - jt], tl[n_time - 1 - jt]
             skip_t = None if last else saved_t[n_time - 2 - jt]
-            yt = self._buf(key, f"dyt{jt}", B * Tin * Ct_in)
-            self._gemm(M=B * Tin, N=2 * Ct_in, Cin=Ct_in, x=xtd, w=W[f"{td}.rewrite.w"], bias=W[f"{td}.rewrite.b"], out=yt,
-                       taps=((0, -1), (0, 0), (0, 1)), I1=1, I0=Tin, J1=1, J0=Tin, xs=(tp4(Tin) * Ct_in, 0, Ct_in, 1),
-                       os_=(Tin * Ct_in, 0, Ct_in), act=_lib.ACT_GLU)
-            nxt_t = self._buf(key, f"tdx{jt}", B * tp4(Tout) * Ct, zero=True)
-            three = tc and 4 * Ct >= 64
-            self._gemm(M=B * (Tin + (0 if three else 1)), N=4 * Ct, Cin=Ct_in, x=yt,
-                       w=W[f"{td}.conv_tr.w3" if three else f"{td}.conv_tr.w"], bias=W[f"{td}.conv_tr.b"], out=nxt_t,
-                       taps=((0, -1), (0, 0), (0, 1)) if three else ((0, 0), (0, -1)), I1=1,
-                       I0=Tin + (0 if three else 1), J1=1, J0=Tin, xs=(Tin * Ct_in, 0, Ct_in, 1),
-                       os_=(tp4(Tout) * Ct, 0, Ct), convt=2 if three else 1, O0=Tout,
-                       act=_lib.ACT_NONE if last else _lib.ACT_GELU, addend=skip_t)
-            if taps is not None:
-                tap(f"tdec{jt}", (nxt_t - skip_t if skip_t is not None else nxt_t).view(B, tp4(Tout), Ct)[:, :Tout], "t")
+            nxt_t = self._buf(key, f"tdx{jt}", B * _pitch(Tout) * Ct, zero=True)
+            self._time_decoder(key, jt, xtd, f"dyt{jt}", nxt_t, skip_t, taps, B, Tin, Tout, Ct_in, Ct)
             xtd = nxt_t
 
         # ---- K2: de-normalise, iSTFT + overlap-add, crop, add the time branch (hdemucs.py:775-793) -----------------
-        if out_buf is not None:
-            if out_buf.numel() != B * S * A * L or out_buf.dtype != torch.float32 or out_buf.device != self.device \
-                    or not out_buf.is_contiguous():
-                raise ValueError("out must be a contiguous float32 tensor of B*S*C*L elements on the engine's device")
-            out = out_buf.view(B, S, A, L)
-        else:
-            out = torch.empty(B, S, A, L, dtype=torch.float32, device=self.device)
-        self._k("bd_istft_ola", ptr(xd), ptr(norm), ptr(self.window), ptr(self.twiddle), ptr(xtd), ptr(out), B, S, T, tp4(L), L,
-                st, nbytes=4.0 * B * S * (T * 2048 * 4 + 2 * L + 2 * L), flops=2.5 * 4096 * 12 * 2 * S * B * T)
-        return out
+        return self._istft(xd, xtd, norm, out_buf, B, T, L, L)
