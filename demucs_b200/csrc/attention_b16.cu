@@ -11,10 +11,9 @@
 // TMEM (512 columns): X3  [S0|P0hi 128][P0lo 64][S1|P1hi 128][P1lo 64][O0 64][O1 64]
 //                     else [S0|P0 128][S1|P1 128][O0 64][O1 64]
 // Replaces the SDPA core of nn.MultiheadAttention (reference transformer.py:365,506).
-#include <cuda.h>
 #include <math.h>
 #include <stdlib.h>
-#include "common.cuh"
+#include "tcgen05.cuh"
 #include "../../include/demucs_b200.h"
 
 namespace {
@@ -22,7 +21,6 @@ namespace {
 constexpr int AT_THREADS = 320;                  // warp 0 TMA, warp 1 MMA, warps 2-5 / 6-9 the two softmax groups
 constexpr int TQ = 128, HD = 64, TK = 128;
 constexpr int TILE = 128 * HD * 2;               // one 128-row x 64-bf16 swizzled box = 16 KB (Q, K and V tiles alike)
-constexpr uint32_t kSpinLimit = 1u << 26;
 constexpr int XCH_LD = 36;                       // floats per row of the final exchange buffer
 
 template <bool X3>
@@ -33,121 +31,6 @@ struct BCfg {
   static constexpr int kSmem = kQBytes + NS * (kKBytes + kVBytes) + 1024 + 512;
   static_assert(NS * kKBytes >= 2 * TQ * XCH_LD * 4, "exchange buffer reuses the K stages");
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) return;
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_3d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void umma_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-               "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-               ::"r"(d), "l"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_ts(uint32_t d, uint32_t a_tmem, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-               "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-               ::"r"(d), "r"(a_tmem), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-// SWIZZLE_128B operand tile of 128-byte rows (64 bf16): SBO = 1024 B between 8-row groups.  The same descriptor
-// serves K-major operands (Q, K: row = query / key, the 64 head dims along K) and the MN-major B operand V
-// (row = key = K index, the 64 head dims along N); the instruction descriptor says which.
-__device__ __forceinline__ uint64_t desc_sw128(const void* smem) {
-  return (uint64_t)((smem_u32(smem) & 0x3FFFF) >> 4) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-         ((uint64_t)2 << 61);
-}
-__host__ __device__ constexpr uint32_t idesc_bf16(int M, int N, int b_mn_major) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) |
-         ((uint32_t)(M >> 4) << 24);
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
-        "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
-        "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-// two floats -> packed bf16x2 (round to nearest even), `a` in the low half (the lower k index)
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  uint32_t r;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
-  return r;
-}
 
 template <bool X3, bool O16>
 __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
@@ -187,15 +70,15 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
     mbar_init(&p_full[1], 128);
     mbar_init(&o_final[0], 1);
     mbar_init(&o_final[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+    tcgen05_alloc(tmem_slot, 512);
+    tcgen05_relinquish();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after();
   const uint32_t tmem = *tmem_slot;
 
   if (warp == 0) {
@@ -222,12 +105,12 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
   } else if (warp == 1) {
     // ===== MMA issuer =====
     if (lane == 0) {
-      constexpr uint32_t idesc_qk = idesc_bf16(TQ, TK, 0);
-      constexpr uint32_t idesc_pv = idesc_bf16(TQ, HD, 1);      // V: MN-major B operand
+      constexpr uint32_t idesc_qk = make_idesc_bf16(TQ, TK);
+      constexpr uint32_t idesc_pv = make_idesc_bf16(TQ, HD, 1);      // V: MN-major B operand
       auto issue_qk = [&](int j) {
         const int s = j % NS, g = j & 1;
         mbar_wait(&k_full[s], (uint32_t)((j / NS) & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         const uint32_t d = tmem + col_s(g);
         const uint8_t* kb = sK + s * kKBytes;
 #pragma unroll
@@ -238,15 +121,15 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
           if (X3) {
             const uint64_t a_lo = desc_sw128(sQ + TILE) + off;
             const uint64_t b_lo = desc_sw128(kb + TILE) + off;
-            umma_ss(d, a_lo, b_hi, idesc_qk, kk != 0);
-            umma_ss(d, a_hi, b_lo, idesc_qk, 1);
-            umma_ss(d, a_hi, b_hi, idesc_qk, 1);
+            umma_bf16(d, a_lo, b_hi, idesc_qk, kk != 0);
+            umma_bf16(d, a_hi, b_lo, idesc_qk, 1);
+            umma_bf16(d, a_hi, b_hi, idesc_qk, 1);
           } else {
-            umma_ss(d, a_hi, b_hi, idesc_qk, kk != 0);
+            umma_bf16(d, a_hi, b_hi, idesc_qk, kk != 0);
           }
         }
-        tc_commit(&s_full[g]);
-        tc_commit(&k_empty[s]);
+        tcgen05_commit(&s_full[g]);
+        tcgen05_commit(&k_empty[s]);
       };
       mbar_wait(q_full, 0);
       issue_qk(0);
@@ -254,9 +137,9 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
       for (int j = 0; j < ntiles; ++j) {
         const int s = j % NS, g = j & 1, i = j >> 1;
         mbar_wait(&p_full[g], (uint32_t)(i & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         mbar_wait(&v_full[s], (uint32_t)((j / NS) & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         const uint8_t* vb = sV + s * kVBytes;
 #pragma unroll
         for (int kk = 0; kk < TK / 16; ++kk) {   // k-steps of 16 keys = 16 rows of V = 2048 bytes; 8 TMEM columns of P
@@ -264,15 +147,15 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
           const uint32_t acc = (i | kk) != 0;
           if (X3) {
             const uint64_t b_lo = desc_sw128(vb + TILE) + (uint32_t)(kk * 128);
-            umma_ts(tmem + col_o(g), tmem + col_plo(g) + kk * 8, b_hi, idesc_pv, acc);
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_lo, idesc_pv, 1);
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, 1);
+            umma_bf16_ts(tmem + col_o(g), tmem + col_plo(g) + kk * 8, b_hi, idesc_pv, acc);
+            umma_bf16_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_lo, idesc_pv, 1);
+            umma_bf16_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, 1);
           } else {
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, acc);
+            umma_bf16_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, acc);
           }
         }
-        tc_commit(&v_empty[s]);
-        if (j + 2 >= ntiles) tc_commit(&o_final[g]);
+        tcgen05_commit(&v_empty[s]);
+        if (j + 2 >= ntiles) tcgen05_commit(&o_final[g]);
         else issue_qk(j + 2);                    // in order behind P V(j): it overwrites the S/P columns of group g
       }
     }
@@ -291,7 +174,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
     for (int j = g; j < ntiles; j += 2, ++i) {
       const int kv_valid = min(TK, Tk - j * TK);
       mbar_wait(&s_full[g], (uint32_t)(i & 1));  // also: every earlier P V of this group has drained
-      tc_fence_after();
+      tcgen05_fence_after();
       // pass 1: row maximum
       float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
 #pragma unroll
@@ -316,7 +199,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
       const float m_cand = fmaxf(fmaxf(mx0, mx1), fmaxf(mx2, mx3)) * sl2;
       const bool raise = m_cand > m_run + 8.0f;   // lazy: P stays below 2^8 with a stale maximum
       if (__any_sync(0xffffffffu, raise)) {
-        const float corr = raise ? ex2_approx(m_run - m_cand) : 1.0f;   // first tile: exp2(-inf) = 0
+        const float corr = raise ? bd_ex2_approx(m_run - m_cand) : 1.0f;   // first tile: exp2(-inf) = 0
         if (i > 0) {
 #pragma unroll
           for (int c0 = 0; c0 < HD; c0 += 32) {
@@ -346,8 +229,8 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
         for (int c = 0; c < 32; c += 4) {
           const float x0 = fmaf(__uint_as_float(v[c]), sl2, -m_run), x1 = fmaf(__uint_as_float(v[c + 1]), sl2, -m_run);
           const float x2 = fmaf(__uint_as_float(v[c + 2]), sl2, -m_run), x3 = fmaf(__uint_as_float(v[c + 3]), sl2, -m_run);
-          float p0 = ex2_approx(x0), p1 = ex2_approx(x1);
-          float p2 = ex2_approx(x2), p3 = ex2_approx(x3);
+          float p0 = bd_ex2_approx(x0), p1 = bd_ex2_approx(x1);
+          float p2 = bd_ex2_approx(x2), p3 = bd_ex2_approx(x3);
           if (kv_valid < TK) {
             if (c0 + c >= kv_valid) p0 = 0.f;
             if (c0 + c + 1 >= kv_valid) p1 = 0.f;
@@ -355,12 +238,12 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
             if (c0 + c + 3 >= kv_valid) p3 = 0.f;
           }
           rs0 += p0; rs1 += p1; rs2 += p2; rs3 += p3;
-          const uint32_t h01 = pack_bf16(p0, p1), h23 = pack_bf16(p2, p3);
+          const uint32_t h01 = bd_pack_bf16(p0, p1), h23 = bd_pack_bf16(p2, p3);
           hi[c >> 1] = h01;
           hi[(c >> 1) + 1] = h23;
           if (X3) {
-            lo[c >> 1] = pack_bf16(p0 - __uint_as_float(h01 << 16), p1 - __uint_as_float(h01 & 0xffff0000u));
-            lo[(c >> 1) + 1] = pack_bf16(p2 - __uint_as_float(h23 << 16), p3 - __uint_as_float(h23 & 0xffff0000u));
+            lo[c >> 1] = bd_pack_bf16(p0 - __uint_as_float(h01 << 16), p1 - __uint_as_float(h01 & 0xffff0000u));
+            lo[(c >> 1) + 1] = bd_pack_bf16(p2 - __uint_as_float(h23 << 16), p3 - __uint_as_float(h23 & 0xffff0000u));
           }
         }
         tmem_st16(s_addr + (c0 >> 1), hi);        // P (hi) over consumed S columns
@@ -369,14 +252,14 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
       }
       tmem_st_wait();
       l_run += (rs0 + rs1) + (rs2 + rs3);
-      tc_fence_before();
+      tcgen05_fence_before();
       mbar_arrive(&p_full[g]);
     }
     // ===== merge the two groups' partial results; group g writes head-dim columns [32g, 32g+32) =====
     float own[32], other[32];
     if (i > 0) {
       mbar_wait(&o_final[g], 0);
-      tc_fence_after();
+      tcgen05_fence_after();
       uint32_t w[HD];
       tmem_ld32_nowait(o_addr, w);
       tmem_ld32_nowait(o_addr + 32, w + 32);
@@ -403,8 +286,8 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
     asm volatile("bar.sync 1, 256;" ::: "memory");
     const float m_o = theirs[32], l_o = theirs[33];
     const float m = fmaxf(m_run, m_o);
-    const float w_s = l_run > 0.f ? ex2_approx(m_run - m) : 0.f;
-    const float w_o = l_o > 0.f ? ex2_approx(m_o - m) : 0.f;
+    const float w_s = l_run > 0.f ? bd_ex2_approx(m_run - m) : 0.f;
+    const float w_o = l_o > 0.f ? bd_ex2_approx(m_o - m) : 0.f;
     const float inv = 1.0f / (l_run * w_s + l_o * w_o);
     const float a_s = w_s * inv, a_o = w_o * inv;
     const int r = q0 + row;
@@ -415,10 +298,10 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
 #pragma unroll
         for (int c = 0; c < 32; c += 8) {
           const float4 t0 = *reinterpret_cast<const float4*>(theirs + c), t1 = *reinterpret_cast<const float4*>(theirs + c + 4);
-          dst[c >> 3] = make_uint4(pack_bf16(fmaf(own[c], a_s, t0.x * a_o), fmaf(own[c + 1], a_s, t0.y * a_o)),
-                                   pack_bf16(fmaf(own[c + 2], a_s, t0.z * a_o), fmaf(own[c + 3], a_s, t0.w * a_o)),
-                                   pack_bf16(fmaf(own[c + 4], a_s, t1.x * a_o), fmaf(own[c + 5], a_s, t1.y * a_o)),
-                                   pack_bf16(fmaf(own[c + 6], a_s, t1.z * a_o), fmaf(own[c + 7], a_s, t1.w * a_o)));
+          dst[c >> 3] = make_uint4(bd_pack_bf16(fmaf(own[c], a_s, t0.x * a_o), fmaf(own[c + 1], a_s, t0.y * a_o)),
+                                   bd_pack_bf16(fmaf(own[c + 2], a_s, t0.z * a_o), fmaf(own[c + 3], a_s, t0.w * a_o)),
+                                   bd_pack_bf16(fmaf(own[c + 4], a_s, t1.x * a_o), fmaf(own[c + 5], a_s, t1.y * a_o)),
+                                   bd_pack_bf16(fmaf(own[c + 6], a_s, t1.z * a_o), fmaf(own[c + 7], a_s, t1.w * a_o)));
         }
       } else {
         float4* dst = reinterpret_cast<float4*>(reinterpret_cast<float*>(ov) + at);
@@ -431,37 +314,21 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_b16_kernel(
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem, 512);
   }
 }
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 // bf16 [B, T, ld] (columns 0 .. D-1 from `base`) -> boxes of 128 rows x 64 columns, SWIZZLE_128B
 bool make_map_b16(CUtensorMap* map, const void* base, int D, int T, int B, int ld = 0) {
   if (!ld) ld = D;
-  static EncodeTiledFn enc = nullptr;
-  if (!enc) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return false;
-    enc = (EncodeTiledFn)p;
-  }
-  cuuint64_t dim[3] = {(cuuint64_t)D, (cuuint64_t)T, (cuuint64_t)B};
-  cuuint64_t str[2] = {(cuuint64_t)ld * 2, (cuuint64_t)T * ld * 2};
-  cuuint32_t box[3] = {64, 128, 1};
-  cuuint32_t es[3] = {1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, (void*)base, dim, str, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  const cuuint64_t dim[3] = {(cuuint64_t)D, (cuuint64_t)T, (cuuint64_t)B};
+  const cuuint64_t str[2] = {(cuuint64_t)ld * 2, (cuuint64_t)T * ld * 2};
+  const cuuint32_t box[3] = {64, 128, 1};
+  return encode_tensor_map(map, base, 3, dim, str, box, 128, true);
 }
 
 // x [rows, ld] (columns 0 .. D-1, fp32) -> dense bf16 hi (and lo = bf16(x - hi)) [rows, D]
@@ -478,8 +345,8 @@ __global__ void split_rows_b16_kernel(const float* __restrict__ x, uint16_t* __r
     uint32_t h[4], l[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      h[k] = pack_bf16(v[2 * k], v[2 * k + 1]);
-      if (X3) l[k] = pack_bf16(v[2 * k] - __uint_as_float(h[k] << 16), v[2 * k + 1] - __uint_as_float(h[k] & 0xffff0000u));
+      h[k] = bd_pack_bf16(v[2 * k], v[2 * k + 1]);
+      if (X3) l[k] = bd_pack_bf16(v[2 * k] - __uint_as_float(h[k] << 16), v[2 * k + 1] - __uint_as_float(h[k] & 0xffff0000u));
     }
     *reinterpret_cast<uint4*>(hi + r * D + c) = make_uint4(h[0], h[1], h[2], h[3]);
     if (X3) *reinterpret_cast<uint4*>(lo + r * D + c) = make_uint4(l[0], l[1], l[2], l[3]);
@@ -544,7 +411,7 @@ int bd_attention_b16(const float* q, const float* k, const float* v, float* o, i
     m[5] = m[2];
   }
   if (!ok) {
-    bd_set_error("bd_attention_b16: cuTensorMapEncodeTiled failed");
+    bd_set_error("bd_attention_b16: TMA tensor map encoding failed");
     return BD_ERR_CUDA;
   }
   return x3 ? launch_attention_b16<true, false>(m, o, B, H, Tq, Tk, ldo, st)
@@ -560,7 +427,7 @@ extern "C" int bd_attention_bf16(const void* q, const void* k, const void* v, vo
   const int D = H * HD;
   alignas(64) CUtensorMap m[6];
   if (!(make_map_b16(&m[0], q, D, Tq, B, ldq) && make_map_b16(&m[1], k, D, Tk, B, ldk) && make_map_b16(&m[2], v, D, Tk, B, ldv))) {
-    bd_set_error("bd_attention_bf16: cuTensorMapEncodeTiled failed");
+    bd_set_error("bd_attention_bf16: TMA tensor map encoding failed");
     return BD_ERR_CUDA;
   }
   m[3] = m[0];

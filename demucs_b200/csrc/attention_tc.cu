@@ -19,10 +19,9 @@
 // so that both parts fit.  TMEM: [S0|P0 .. 128][S1|P1 .. 128][O0 64][O1 64].
 // Token counts are not multiples of the tile: TMA zero-fills rows past the item, the softmax masks them.
 // Replaces the SDPA core of nn.MultiheadAttention (reference transformer.py:365,506).
-#include <cuda.h>
 #include <math.h>
 #include <stdlib.h>
-#include "common.cuh"
+#include "tcgen05.cuh"
 #include "../../include/demucs_b200.h"
 
 namespace {
@@ -31,7 +30,6 @@ constexpr int AT_THREADS = 320;                  // warp 0 TMA, warp 1 MMA, warp
 constexpr int TQ = 128, HD = 64;
 constexpr int SUB = TQ * 32 * 4;                 // one 128-row x 32-float swizzled box = 16 KB
 constexpr int VSUB = HD * 32 * 4;                // one 64-row x 32-float box of V^T = 8 KB
-constexpr uint32_t kSpinLimit = 1u << 26;
 constexpr int XCH_LD = 36;                       // floats per row of the final exchange buffer
 
 template <bool X3>
@@ -46,110 +44,6 @@ struct ACfg {
   static constexpr int kSmem = kQBytes + NS * (kKBytes + kVBytes) + 1024 + 512;
   static_assert(NS * kKBytes >= 2 * TQ * XCH_LD * 4, "exchange buffer reuses the K stages");
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) return;
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_3d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void tc_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-
-__device__ __forceinline__ void umma_ss(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-               "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-               ::"r"(d), "l"(a), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_ts(uint32_t d, uint32_t a_tmem, uint64_t b, uint32_t idesc, uint32_t acc) {
-  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-               "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-               ::"r"(d), "r"(a_tmem), "l"(b), "r"(idesc), "r"(acc) : "memory");
-}
-// K-major SWIZZLE_128B operand (rows of 32 floats): SBO = 1024 B between 8-row groups
-__device__ __forceinline__ uint64_t desc_kmajor(const void* smem) {
-  return (uint64_t)((smem_u32(smem) & 0x3FFFF) >> 4) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-         ((uint64_t)2 << 61);
-}
-__host__ __device__ constexpr uint32_t idesc_tf32(int M, int N, int b_mn_major) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) |
-         ((uint32_t)(M >> 4) << 24);
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_st32(uint32_t taddr, const uint32_t* r) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-      "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-        "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
-        "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
-        "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld32_nowait(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ float ex2_approx(float x) {
-  float y;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-__device__ __forceinline__ float tf32_rna(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return __uint_as_float(r);
-}
-__device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 template <bool X3>
 __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
@@ -189,15 +83,15 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
     mbar_init(&p_full[1], 128);
     mbar_init(&o_final[0], 1);
     mbar_init(&o_final[1], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+    tcgen05_alloc(tmem_slot, 512);
+    tcgen05_relinquish();
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
-  tc_fence_after();
+  tcgen05_fence_after();
   const uint32_t tmem = *tmem_slot;
 
   if (warp == 0) {
@@ -233,31 +127,31 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
   } else if (warp == 1) {
     // ===== MMA issuer =====
     if (lane == 0) {
-      constexpr uint32_t idesc_qk = idesc_tf32(TQ, TK, 0);
-      constexpr uint32_t idesc_pv = idesc_tf32(TQ, HD, 0);
+      constexpr uint32_t idesc_qk = make_idesc_tf32(TQ, TK);
+      constexpr uint32_t idesc_pv = make_idesc_tf32(TQ, HD);
       auto issue_qk = [&](int j) {
         const int s = j % NS, g = j & 1;
         mbar_wait(&k_full[s], (uint32_t)((j / NS) & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         const uint32_t d = tmem + col_s(g);
         const uint8_t* kb = sK + s * kKBytes;
 #pragma unroll
         for (int kk = 0; kk < HD / 8; ++kk) {   // 8 k-steps: two 32-float boxes x 4
           const uint32_t x = kk >> 2, off = 2 * (kk & 3);
-          const uint64_t a_hi = desc_kmajor(sQ + x * SUB) + off;
-          const uint64_t b_hi = desc_kmajor(kb + x * KSUB) + off;
+          const uint64_t a_hi = desc_sw128(sQ + x * SUB) + off;
+          const uint64_t b_hi = desc_sw128(kb + x * KSUB) + off;
           if (X3) {
-            const uint64_t a_lo = desc_kmajor(sQ + (2 + x) * SUB) + off;
-            const uint64_t b_lo = desc_kmajor(kb + (2 + x) * KSUB) + off;
-            umma_ss(d, a_lo, b_hi, idesc_qk, kk != 0);
-            umma_ss(d, a_hi, b_lo, idesc_qk, 1);
-            umma_ss(d, a_hi, b_hi, idesc_qk, 1);
+            const uint64_t a_lo = desc_sw128(sQ + (2 + x) * SUB) + off;
+            const uint64_t b_lo = desc_sw128(kb + (2 + x) * KSUB) + off;
+            umma_tf32(d, a_lo, b_hi, idesc_qk, kk != 0);
+            umma_tf32(d, a_hi, b_lo, idesc_qk, 1);
+            umma_tf32(d, a_hi, b_hi, idesc_qk, 1);
           } else {
-            umma_ss(d, a_hi, b_hi, idesc_qk, kk != 0);
+            umma_tf32(d, a_hi, b_hi, idesc_qk, kk != 0);
           }
         }
-        tc_commit(&s_full[g]);
-        tc_commit(&k_empty[s]);
+        tcgen05_commit(&s_full[g]);
+        tcgen05_commit(&k_empty[s]);
       };
       mbar_wait(q_full, 0);
       issue_qk(0);
@@ -265,26 +159,26 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
       for (int j = 0; j < ntiles; ++j) {
         const int s = j % NS, g = j & 1, i = j >> 1;
         mbar_wait(&p_full[g], (uint32_t)(i & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         mbar_wait(&v_full[s], (uint32_t)((j / NS) & 1));
-        tc_fence_after();
+        tcgen05_fence_after();
         const uint8_t* vb = sV + s * kVBytes;
 #pragma unroll
         for (int kk = 0; kk < TK / 8; ++kk) {   // k-steps of 8 keys
           const uint32_t off = 2 * (kk & 3);
-          const uint64_t b_hi = desc_kmajor(vb + (kk >> 2) * VSUB) + off;
+          const uint64_t b_hi = desc_sw128(vb + (kk >> 2) * VSUB) + off;
           const uint32_t acc = (i | kk) != 0;
           if (X3) {
-            const uint64_t b_lo = desc_kmajor(vb + ((TK / 32) + (kk >> 2)) * VSUB) + off;
-            umma_ts(tmem + col_o(g), tmem + col_plo(g) + kk * 8, b_hi, idesc_pv, acc);
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_lo, idesc_pv, 1);
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, 1);
+            const uint64_t b_lo = desc_sw128(vb + ((TK / 32) + (kk >> 2)) * VSUB) + off;
+            umma_tf32_ts(tmem + col_o(g), tmem + col_plo(g) + kk * 8, b_hi, idesc_pv, acc);
+            umma_tf32_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_lo, idesc_pv, 1);
+            umma_tf32_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, 1);
           } else {
-            umma_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, acc);
+            umma_tf32_ts(tmem + col_o(g), tmem + col_s(g) + kk * 8, b_hi, idesc_pv, acc);
           }
         }
-        tc_commit(&v_empty[s]);
-        if (j + 2 >= ntiles) tc_commit(&o_final[g]);
+        tcgen05_commit(&v_empty[s]);
+        if (j + 2 >= ntiles) tcgen05_commit(&o_final[g]);
         else issue_qk(j + 2);                    // in order behind P V(j): it overwrites the S/P columns of group g
       }
     }
@@ -302,7 +196,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
     for (int j = g; j < ntiles; j += 2, ++i) {
       const int kv_valid = min(TK, Tk - j * TK);
       mbar_wait(&s_full[g], (uint32_t)(i & 1));  // also: every earlier P V of this group has drained
-      tc_fence_after();
+      tcgen05_fence_after();
       // pass 1: row maximum (the S row is read again, chunk by chunk, in pass 2: tensor memory is cheap to read
       // and 128 live values would not leave room for anything else)
       float mx0 = -INFINITY, mx1 = -INFINITY, mx2 = -INFINITY, mx3 = -INFINITY;
@@ -328,7 +222,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
       const float m_cand = fmaxf(fmaxf(mx0, mx1), fmaxf(mx2, mx3)) * sl2;
       const bool raise = m_cand > m_run + 8.0f;   // lazy: P stays below 2^8 with a stale maximum
       if (__any_sync(0xffffffffu, raise)) {
-        const float corr = raise ? ex2_approx(m_run - m_cand) : 1.0f;   // first tile: exp2(-inf) = 0
+        const float corr = raise ? bd_ex2_approx(m_run - m_cand) : 1.0f;   // first tile: exp2(-inf) = 0
         if (i > 0) {
 #pragma unroll
           for (int c0 = 0; c0 < HD; c0 += 32) {
@@ -357,8 +251,8 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
         for (int c = 0; c < 32; c += 4) {
           const float x0 = fmaf(__uint_as_float(v[c]), sl2, -m_run), x1 = fmaf(__uint_as_float(v[c + 1]), sl2, -m_run);
           const float x2 = fmaf(__uint_as_float(v[c + 2]), sl2, -m_run), x3 = fmaf(__uint_as_float(v[c + 3]), sl2, -m_run);
-          float p0 = ex2_approx(x0), p1 = ex2_approx(x1);
-          float p2 = ex2_approx(x2), p3 = ex2_approx(x3);
+          float p0 = bd_ex2_approx(x0), p1 = bd_ex2_approx(x1);
+          float p2 = bd_ex2_approx(x2), p3 = bd_ex2_approx(x3);
           if (kv_valid < TK) {
             if (c0 + c >= kv_valid) p0 = 0.f;
             if (c0 + c + 1 >= kv_valid) p1 = 0.f;
@@ -367,7 +261,7 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
           }
           rs0 += p0; rs1 += p1; rs2 += p2; rs3 += p3;
           if (X3) {
-            const float h0 = tf32_rna(p0), h1 = tf32_rna(p1), h2 = tf32_rna(p2), h3 = tf32_rna(p3);
+            const float h0 = bd_tf32_rna(p0), h1 = bd_tf32_rna(p1), h2 = bd_tf32_rna(p2), h3 = bd_tf32_rna(p3);
             v[c] = __float_as_uint(h0); v[c + 1] = __float_as_uint(h1);
             v[c + 2] = __float_as_uint(h2); v[c + 3] = __float_as_uint(h3);
             lo[c] = __float_as_uint(p0 - h0); lo[c + 1] = __float_as_uint(p1 - h1);
@@ -383,14 +277,14 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
       }
       tmem_st_wait();
       l_run += (rs0 + rs1) + (rs2 + rs3);
-      tc_fence_before();
+      tcgen05_fence_before();
       mbar_arrive(&p_full[g]);
     }
     // ===== merge the two groups' partial results; group g writes head-dim columns [32g, 32g+32) =====
     float own[32], other[32];
     if (i > 0) {
       mbar_wait(&o_final[g], 0);
-      tc_fence_after();
+      tcgen05_fence_after();
       uint32_t w[HD];
       tmem_ld32_nowait(o_addr, w);
       tmem_ld32_nowait(o_addr + 32, w + 32);
@@ -417,8 +311,8 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
     asm volatile("bar.sync 1, 256;" ::: "memory");
     const float m_o = theirs[32], l_o = theirs[33];
     const float m = fmaxf(m_run, m_o);
-    const float w_s = l_run > 0.f ? ex2_approx(m_run - m) : 0.f;
-    const float w_o = l_o > 0.f ? ex2_approx(m_o - m) : 0.f;
+    const float w_s = l_run > 0.f ? bd_ex2_approx(m_run - m) : 0.f;
+    const float w_o = l_o > 0.f ? bd_ex2_approx(m_o - m) : 0.f;
     const float inv = 1.0f / (l_run * w_s + l_o * w_o);
     const float a_s = w_s * inv, a_o = w_o * inv;
     const int r = q0 + row;
@@ -432,36 +326,22 @@ __global__ void __launch_bounds__(AT_THREADS, 1) attention_tc_kernel(
       }
     }
   }
-  tc_fence_before();
+  tcgen05_fence_before();
   __syncthreads();
   if (warp == 1) {
-    tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
+    tcgen05_fence_after();
+    tcgen05_dealloc(tmem, 512);
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
+// fp32 [B, T, ld] (columns 0 .. cols-1 from `base`, items `item_stride` floats apart, default T * ld) -> boxes of
+// box_rows rows x 32 columns, SWIZZLE_128B
 bool make_map3(CUtensorMap* map, const float* base, int cols, int T, int B, int ld, int box_rows = 128,
                long long item_stride = 0) {
-  static EncodeTiledFn enc = nullptr;
-  if (!enc) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return false;
-    enc = (EncodeTiledFn)p;
-  }
-  cuuint64_t dim[3] = {(cuuint64_t)cols, (cuuint64_t)T, (cuuint64_t)B};
-  cuuint64_t str[2] = {(cuuint64_t)ld * 4, (cuuint64_t)(item_stride ? item_stride : (long long)T * ld) * 4};
-  cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
-  cuuint32_t es[3] = {1, 1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*)base, dim, str, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-             CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+  const cuuint64_t dim[3] = {(cuuint64_t)cols, (cuuint64_t)T, (cuuint64_t)B};
+  const cuuint64_t str[2] = {(cuuint64_t)ld * 4, (cuuint64_t)(item_stride ? item_stride : (long long)T * ld) * 4};
+  const cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
+  return encode_tensor_map(map, base, 3, dim, str, box, 128);
 }
 
 // v [B, Tk, ldv] (columns 0 .. D-1) -> vt [B, D, Tkp], 32x32 tiles through shared memory.  SPLIT: write the
@@ -483,7 +363,7 @@ __global__ void transpose_v_kernel(const float* __restrict__ v, float* __restric
       const float x = tile[tx][i];
       const size_t at = ((size_t)b * D + c0 + i) * Tkp + t;
       if (SPLIT) {
-        const float hi = tf32_rna(x);
+        const float hi = bd_tf32_rna(x);
         vt[at] = hi;
         vt_lo[at] = x - hi;
       } else {
@@ -501,7 +381,7 @@ __global__ void split_rows_kernel(const float* __restrict__ x, float* __restrict
     const long long r = i / (D / 4);
     const int c = (int)(i - r * (D / 4)) * 4;
     const float4 t = __ldg(reinterpret_cast<const float4*>(x + r * ld + c));
-    const float4 h = make_float4(tf32_rna(t.x), tf32_rna(t.y), tf32_rna(t.z), tf32_rna(t.w));
+    const float4 h = make_float4(bd_tf32_rna(t.x), bd_tf32_rna(t.y), bd_tf32_rna(t.z), bd_tf32_rna(t.w));
     *reinterpret_cast<float4*>(hi + r * D + c) = h;
     *reinterpret_cast<float4*>(lo + r * D + c) = make_float4(t.x - h.x, t.y - h.y, t.z - h.z, t.w - h.w);
   }
@@ -568,7 +448,7 @@ int bd_attention_tc(const float* q, const float* k, const float* v, float* o, in
     m[5] = m[2];
   }
   if (!ok) {
-    bd_set_error("bd_attention_tc: cuTensorMapEncodeTiled failed");
+    bd_set_error("bd_attention_tc: TMA tensor map encoding failed");
     return BD_ERR_CUDA;
   }
   return x3 ? launch_attention<true>(m, o, B, H, Tq, Tk, ldo, st) : launch_attention<false>(m, o, B, H, Tq, Tk, ldo, st);

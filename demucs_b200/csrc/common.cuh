@@ -26,6 +26,25 @@ __device__ __forceinline__ float bd_gelu(float x) {
 }
 // ex2.approx + rcp.approx: ~2 ulp, a handful of instructions (an IEEE division costs ~40 in a GEMM epilogue)
 __device__ __forceinline__ float bd_sigmoid(float x) { return __fdividef(1.0f, 1.0f + __expf(-x)); }
+__device__ __forceinline__ float bd_ex2_approx(float x) {
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+
+// two floats -> packed bf16x2 (round to nearest even), `a` in the low half (the lower address / lower k index)
+__device__ __forceinline__ uint32_t bd_pack_bf16(float a, float b) {
+  uint32_t r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
+  return r;
+}
+// round-to-nearest TF32 (low 13 mantissa bits cleared): exactly representable, so the tensor core's own
+// fp32 -> tf32 conversion of it is the identity
+__device__ __forceinline__ float bd_tf32_rna(float x) {
+  uint32_t r;
+  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
+  return __uint_as_float(r);
+}
 
 __device__ __forceinline__ float bd_warp_sum(float v) {
 #pragma unroll

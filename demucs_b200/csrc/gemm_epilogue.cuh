@@ -58,11 +58,6 @@ __device__ __forceinline__ long long bd_col_ofs(const bd_gemm_desc& d, int no) {
 }
 
 // output stores: fp32, or bf16 (round to nearest even) when the descriptor says the output tensor is bf16
-__device__ __forceinline__ uint32_t bd_pack_bf16(float a, float b) {
-  uint32_t r;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
-  return r;
-}
 __device__ __forceinline__ void bd_store_out4(const bd_gemm_desc& d, long long o, float4 v) {
   if (d.out_bf16)
     *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(d.out) + o) = make_uint2(bd_pack_bf16(v.x, v.y), bd_pack_bf16(v.z, v.w));

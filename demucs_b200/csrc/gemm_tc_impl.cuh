@@ -12,7 +12,7 @@
 // running at the same time share the activation rows in L2):
 //   warp 0      TMA producer (one elected lane); the shared-memory ring (4..16 stages) never drains between tiles
 //   warp 1      TMEM allocator + MMA issuer (one elected lane)
-//   warps 4..7  (3xTF32) operand splitter: x -> rn_tf32(x), x - rn_tf32(x) in shared memory (bf16 modes: warps 2..)
+//   warps 4..7  (3xTF32) operand splitter: x -> bd_tf32_rna(x), x - hi in shared memory (bf16 modes: warps 2..)
 //   last 8..16  epilogue warps, warp w owns TMEM lanes 32*(w%4)..+31.  Wide tiles (TBN >= 64): the 2..4 warps of
 //               a lane quarter split the tile's columns and the accumulator is double-buffered, so the epilogue
 //               of tile i runs under the main loop of tile i+1.  Tiles of 96 / 192 / 256 columns are finished in
@@ -54,9 +54,9 @@
 //   MODE 4  BF16D    the same with a bf16 A tensor in HBM: the tile arrives by TMA in operand form (64 elements =
 //                    128-byte rows per k-block), no splitter warps
 #pragma once
-#include <cuda.h>
 #include <stdlib.h>
 #include "gemm_epilogue.cuh"
+#include "tcgen05.cuh"
 
 enum { BD_TC_TF32 = 0, BD_TC_TF32X3 = 1, BD_TC_BF16X3 = 2, BD_TC_BF16 = 3, BD_TC_BF16D = 4 };
 
@@ -74,7 +74,7 @@ constexpr int TBM = 128;                           // tile rows (UMMA M)
 
 // TBK floats per k-block: 32 -> 128B swizzle, 16 -> 64B swizzle.  TBN = tile columns = UMMA N (16..128):
 // narrow outputs (DConv hidden widths, last-layer channels) get narrow tiles instead of zero padding.
-// X3: error-compensated "3xTF32": every operand tile is split in shared memory into hi = rn_tf32(x) and
+// X3: error-compensated "3xTF32": every operand tile is split in shared memory into hi = bd_tf32_rna(x) and
 // lo = x - hi and the product is accumulated as hi*hi + lo*hi + hi*lo (fp32-class accuracy, 3x the MMAs).
 
 struct RowInfo {           // per-row epilogue constants, parked in shared memory (32 bytes)
@@ -85,225 +85,14 @@ struct RowInfo {           // per-row epilogue constants, parked in shared memor
   int pad0, pad1;
 };
 
-constexpr uint32_t kSpinLimit = 1u << 26;          // turn a lost barrier into a trap, never a hang
-
-// ---- PTX wrappers ------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) return;
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-// Single-thread roles (TMA producer, MMA issuer) in the persistent kernel: let the hardware park the thread for
-// up to ~1 us per poll instead of spinning through the issue slots the epilogue warps need.
-__device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity), "r"(1000)
-        : "memory");
-    if (done) return;
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-// Same, for waiters that are not on the critical path (epilogue warps parked during the main loop, the
-// producer waiting for a free stage): back off between polls so that they do not compete for issue slots.
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0, spins = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) return;
-    __nanosleep(64);
-    if (++spins > kSpinLimit) __trap();
-  }
-}
-__device__ __forceinline__ void tma_load_4d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2,
-                                            int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_5d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1, int c2,
-                                            int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], "
-      "[%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap* map, uint64_t* bar, void* dst, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tcgen05_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void tcgen05_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tcgen05_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-
-// D[tmem] (+)= A[smem desc] * B[smem desc], TF32 inputs, fp32 accumulate
-__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-// D[tmem] (+)= A[smem desc] * B[smem desc], BF16 inputs, fp32 accumulate (K = 16 per instruction)
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// D[tmem] (+)= A[tmem] * B[smem desc], BF16 inputs: A is 128 lanes x 8 columns per K = 16 (two bf16 per column)
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout):
-//   [0,14) start>>4 | [16,30) LBO>>4 (unused for swizzled K-major) | [32,46) SBO>>4 = 8 rows * 128 B
-//   [46,48) version = 1 | [61,64) layout = 2 (SWIZZLE_128B)
-//   SWIZZLE_64B (16-float rows): SBO = 8 rows * 64 B, layout = 4
-template <int TBK>
-__device__ __forceinline__ uint64_t make_kmajor_desc(const void* smem) {
-  uint64_t desc = (uint64_t)((smem_u32(smem) & 0x3FFFF) >> 4);
-  desc |= (uint64_t)((8 * TBK * 4) >> 4) << 32;
-  desc |= (uint64_t)1 << 46;
-  desc |= (uint64_t)(TBK == 32 ? 2 : 4) << 61;
-  return desc;
-}
-// K-major descriptor of a 16-bit operand tile whose rows hold TBK elements (64-byte rows: SWIZZLE_64B, 32-byte rows:
-// SWIZZLE_32B); `sbo` = bytes between consecutive 8-row groups (the in-place split A tile interleaves its hi and lo
-// groups, so its groups are twice as far apart as those of a dense tile)
-template <int TBK>
-__device__ __forceinline__ uint64_t make_kmajor_desc16(const void* smem, int sbo) {
-  uint64_t desc = (uint64_t)((smem_u32(smem) & 0x3FFFF) >> 4);
-  desc |= (uint64_t)(sbo >> 4) << 32;
-  desc |= (uint64_t)1 << 46;
-  desc |= (uint64_t)(TBK == 64 ? 2 : TBK == 32 ? 4 : 6) << 61;      // 128 / 64 / 32-byte rows
-  return desc;
-}
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// two floats -> packed bf16x2 (round to nearest even), `a` in the low half (the lower address / lower k index)
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-  uint32_t r;
-  asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
-  return r;
-}
-// Instruction descriptor (cute::UMMA::InstrDescriptor): c=F32, a=b=TF32, both K-major, N, M
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// round-to-nearest TF32 (low 13 mantissa bits cleared): exactly representable, so the tensor core's own
-// fp32 -> tf32 conversion of it is the identity
-__device__ __forceinline__ float rn_tf32(float x) {
-  uint32_t u;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(u) : "f"(x));
-  return __uint_as_float(u);
-}
-
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// this thread's TMEM lane, N consecutive 32-bit columns from `taddr`; returns once the data is in tensor memory
-template <int N>
-__device__ __forceinline__ void tmem_st(uint32_t taddr, const uint32_t* r) {
-  static_assert(N == 16 || N == 32, "tmem_st: 16 or 32 columns");
-  if constexpr (N == 32) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x32.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, "
-        "%17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32};"
-        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-          "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15]), "r"(r[16]), "r"(r[17]),
-          "r"(r[18]), "r"(r[19]), "r"(r[20]), "r"(r[21]), "r"(r[22]), "r"(r[23]), "r"(r[24]), "r"(r[25]), "r"(r[26]),
-          "r"(r[27]), "r"(r[28]), "r"(r[29]), "r"(r[30]), "r"(r[31])
-        : "memory");
-  } else {
-    asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-          "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
-        : "memory");
-  }
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-
 // ---- lean epilogue for the common layer shapes -----------------------------------------------------------
 // The generic bd_epi_* helpers test every optional operand per 4-column group; for the layers that dominate the
 // run time (plain / GELU / GLU, optional GroupNorm affine, optional LayerScale residual; no transposed-conv
 // scatter, channel split, row bias or addend) this version fixes the combination at compile time, keeps
 // everything in 32-bit shared-space addresses and predicates instead of branching on row / column validity.
 __device__ __forceinline__ float sigmoid_fast(float x) {
-  float e, r;
-  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(-1.44269504088896340736f * x));
+  const float e = bd_ex2_approx(-1.44269504088896340736f * x);
+  float r;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.0f + e));
   return r;
 }
@@ -550,12 +339,11 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
       mbar_init(&tmem_full[a], 1);
       mbar_init(&tmem_empty[a], kTileSplit ? 4 : 4 * kPGroups);   // one arrival per epilogue warp of the tile
     }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_fence_init();
   }
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)),
-                 "r"(kTmemCols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
+    tcgen05_alloc(tmem_slot, kTmemCols);
+    tcgen05_relinquish();
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -677,6 +465,7 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
       // floats (16-byte chunks in the TMA swizzle: 8 consecutive rows hit 8 different chunk positions, no bank
       // conflict) and stores bf16 hi | lo into the stage's TMEM slot.  The slot is free once full_bar[s] completes:
       // the producer refilled stage s only after the MMAs that last read the slot committed empty_bar[s].
+      static_assert(TBK == 16 || TBK == 32, "A in tensor memory: 16 or 32 columns per stage");
       constexpr int RB = TBK * 4;                          // bytes per fp32 row
       const int row = 32 * (warp & 3) + lane;
       const int xr = (row * RB >> 7) & (RB / 16 - 1);      // swizzle XOR term of the row
@@ -691,14 +480,16 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
 #pragma unroll
           for (int j = 0; j < TBK / 4; ++j) {
             const float4 x = *reinterpret_cast<const float4*>(rp + ((j ^ xr) << 4));
-            const uint32_t h0 = pack_bf16(x.x, x.y), h1 = pack_bf16(x.z, x.w);
+            const uint32_t h0 = bd_pack_bf16(x.x, x.y), h1 = bd_pack_bf16(x.z, x.w);
             hl[2 * j] = h0;
             hl[2 * j + 1] = h1;
-            hl[TBK / 2 + 2 * j] = pack_bf16(x.x - __uint_as_float(h0 << 16), x.y - __uint_as_float(h0 & 0xffff0000u));
-            hl[TBK / 2 + 2 * j + 1] = pack_bf16(x.z - __uint_as_float(h1 << 16), x.w - __uint_as_float(h1 & 0xffff0000u));
+            hl[TBK / 2 + 2 * j] = bd_pack_bf16(x.x - __uint_as_float(h0 << 16), x.y - __uint_as_float(h0 & 0xffff0000u));
+            hl[TBK / 2 + 2 * j + 1] = bd_pack_bf16(x.z - __uint_as_float(h1 << 16), x.w - __uint_as_float(h1 & 0xffff0000u));
           }
           tcgen05_fence_after();
-          tmem_st<TBK>(tmem_base + lane_addr + (uint32_t)(C_::kACol0 + s * TBK), hl);
+          const uint32_t slot = tmem_base + lane_addr + (uint32_t)(C_::kACol0 + s * TBK);
+          if constexpr (TBK == 32) tmem_st32(slot, hl); else tmem_st16(slot, hl);
+          tmem_st_wait();
           tcgen05_fence_before();
           mbar_arrive(&conv_bar[s]);
         }
@@ -742,13 +533,13 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
 #pragma unroll
             for (int j = 0; j < (TBK == 32 ? 2 : 1); ++j) {
               const float4 x = v[i][j];
-              const uint32_t h0 = pack_bf16(x.x, x.y), h1 = pack_bf16(x.z, x.w);
+              const uint32_t h0 = bd_pack_bf16(x.x, x.y), h1 = bd_pack_bf16(x.z, x.w);
               hi[2 * j] = h0;
               hi[2 * j + 1] = h1;
               lo[2 * j] = lo[2 * j + 1] = 0u;
               if constexpr (MODE == BD_TC_BF16X3) {
-                lo[2 * j] = pack_bf16(x.x - __uint_as_float(h0 << 16), x.y - __uint_as_float(h0 & 0xffff0000u));
-                lo[2 * j + 1] = pack_bf16(x.z - __uint_as_float(h1 << 16), x.w - __uint_as_float(h1 & 0xffff0000u));
+                lo[2 * j] = bd_pack_bf16(x.x - __uint_as_float(h0 << 16), x.y - __uint_as_float(h0 & 0xffff0000u));
+                lo[2 * j + 1] = bd_pack_bf16(x.z - __uint_as_float(h1 << 16), x.w - __uint_as_float(h1 & 0xffff0000u));
               }
             }
             if constexpr (TBK == 32) {
@@ -778,7 +569,7 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
 #pragma unroll 4
           for (int i = et; i < tile_bytes / 16; i += 128) {
             const float4 x = hi[i];
-            const float4 h = make_float4(rn_tf32(x.x), rn_tf32(x.y), rn_tf32(x.z), rn_tf32(x.w));
+            const float4 h = make_float4(bd_tf32_rna(x.x), bd_tf32_rna(x.y), bd_tf32_rna(x.z), bd_tf32_rna(x.w));
             hi[i] = h;
             lo[i] = make_float4(x.x - h.x, x.y - h.y, x.z - h.z, x.w - h.w);
           }
@@ -982,40 +773,11 @@ __global__ void __launch_bounds__((PCfg<TBK, TBN, MODE, ATM>::kThreads), 1) conv
   __syncthreads();
   if (warp == 1) {
     tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols));
+    tcgen05_dealloc(tmem_base, kTmemCols);
   }
 }
 
 // ---- host side ------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-        q != cudaDriverEntryPointSuccess)
-      return nullptr;
-    fn = (EncodeTiledFn)p;
-  }
-  return fn;
-}
-
-bool encode(CUtensorMap* map, const void* base, int rank, const cuuint64_t* gdim, const cuuint64_t* gstride_bytes,
-            const cuuint32_t* box, int row_bytes, bool bf16 = false) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) return false;
-  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  const CUtensorMapSwizzle sw = row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                : row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
-  return enc(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, rank, (void*)base, gdim,
-             gstride_bytes, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 template <int TBK, int TBN, int MODE, bool ATM = false>
 int launch_tc_persist(const bd_gemm_desc& d, const TileGeom& g, int items, cudaStream_t st) {
   using C_ = PCfg<TBK, TBN, MODE, ATM>;
@@ -1034,18 +796,18 @@ int launch_tc_persist(const bd_gemm_desc& d, const TileGeom& g, int items, cudaS
   }
   cuuint64_t bdim[2] = {(cuuint64_t)d.K, (cuuint64_t)d.N};
   cuuint32_t bbox[2] = {(cuuint32_t)TBK, (cuuint32_t)TBN};
-  bool ok = encode(&map_a, d.x, arank, adim, astr, abox, TBK * ES, C_::kDirect);
+  bool ok = encode_tensor_map(&map_a, d.x, arank, adim, astr, abox, TBK * ES, C_::kDirect);
   if constexpr (C_::kB16) {
     cuuint64_t bstr[1] = {(cuuint64_t)d.K * 2};
-    ok = ok && encode(&map_b, d.w16_hi, 2, bdim, bstr, bbox, TBK * 2, true);
-    ok = ok && encode(&map_b_lo, MODE == BD_TC_BF16X3 ? d.w16_lo : d.w16_hi, 2, bdim, bstr, bbox, TBK * 2, true);
+    ok = ok && encode_tensor_map(&map_b, d.w16_hi, 2, bdim, bstr, bbox, TBK * 2, true);
+    ok = ok && encode_tensor_map(&map_b_lo, MODE == BD_TC_BF16X3 ? d.w16_lo : d.w16_hi, 2, bdim, bstr, bbox, TBK * 2, true);
   } else {
     cuuint64_t bstr[1] = {(cuuint64_t)d.K * 4};
-    ok = ok && encode(&map_b, d.w, 2, bdim, bstr, bbox, TBK * 4);
+    ok = ok && encode_tensor_map(&map_b, d.w, 2, bdim, bstr, bbox, TBK * 4);
     map_b_lo = map_b;
   }
   if (!ok) {
-    bd_set_error("bd_conv_gemm_tc: cuTensorMapEncodeTiled failed (M=%d N=%d K=%d Cin=%d J0=%d J1=%d)", d.M, d.N, d.K,
+    bd_set_error("bd_conv_gemm_tc: TMA tensor map encoding failed (M=%d N=%d K=%d Cin=%d J0=%d J1=%d)", d.M, d.N, d.K,
                  d.Cin, d.J0, d.J1);
     return BD_ERR_CUDA;
   }

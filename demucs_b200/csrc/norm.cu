@@ -120,10 +120,7 @@ __global__ void layer_norm_kernel(const float* __restrict__ x, void* __restrict_
         o.x += p.x; o.y += p.y; o.z += p.z; o.w += p.w;
       }
       if (Y16) {
-        uint32_t lo, hi;
-        asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(o.y), "f"(o.x));
-        asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(o.w), "f"(o.z));
-        yh[idx] = make_uint2(lo, hi);
+        yh[idx] = make_uint2(bd_pack_bf16(o.x, o.y), bd_pack_bf16(o.z, o.w));
       } else {
         yr[idx] = o;
       }

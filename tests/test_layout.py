@@ -27,6 +27,25 @@ def test_product_never_imports_the_oracle():
             assert "refload" not in src, fn
 
 
+def test_tensor_core_primitives_live_in_one_header():
+    # the mbarrier / TMA / tcgen05 wrappers, the bf16x2 conversion and the tensor-map encoder are written once
+    # (csrc/tcgen05.cuh, csrc/common.cuh) so that the GEMM and both attention kernels issue them the same way
+    csrc = os.path.join(ROOT, "demucs_b200", "csrc")
+    home = {"mbarrier.": "tcgen05.cuh", "cp.async.bulk.tensor": "tcgen05.cuh", "tcgen05.": "tcgen05.cuh",
+            "cvt.rn.bf16x2": "common.cuh"}
+    for fn in sorted(os.listdir(csrc)):
+        if not fn.endswith((".cu", ".cuh")):
+            continue
+        src = open(os.path.join(csrc, fn)).read()
+        code = re.sub(r"^\s*#\s*include.*$", "", src, flags=re.M)
+        strings = re.findall(r'"(?:[^"\\\n]|\\.)*"', code)   # quoted strings only: comments may name instructions
+        for op, owner in home.items():
+            if fn != owner:
+                assert not [s for s in strings if op in s], f"{fn}: {op} outside {owner}"
+        if fn != "tcgen05.cuh":
+            assert "cuTensorMapEncodeTiled" not in src, fn
+
+
 def test_gemm_desc_mirror_matches_header_field_order():
     header = open(os.path.join(ROOT, "include", "demucs_b200.h")).read()
     body = header[header.index("typedef struct bd_gemm_desc {"):header.index("} bd_gemm_desc;")]
