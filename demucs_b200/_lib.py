@@ -84,6 +84,7 @@ SIGNATURES: tp.Dict[str, tp.List] = {
     "bd_resample_frac": [_P, _P, _P, _I, _I, _I, _LL, _LL, _I, _I, _I, _P],
     "bd_absmax": [_P, _P, _LL, _P],
     "bd_clip_pcm": [_P, _P, _I, _LL, _I, _P, _I, _P],
+    "bd_pcm_decode": [_P, _P, _I, _I, _I, _LL, _LL, _LL, _P],
 }
 VALUE_CALLS = {"bd_attention_workspace"}          # entry points that return a value, not a status
 EXPORTS = ["bd_last_error", "bd_version"] + list(SIGNATURES)

@@ -8,7 +8,8 @@ names the random-init stand-ins of the released architectures, and a model objec
 Audio that is not at the model's sample rate / channel count is converted on the device
 (``demucs_b200.audio.convert_audio``, the julius-equivalent polyphase resampler), and
 ``separate_tensor_pcm`` / ``demucs_b200.audio.save_audio`` take the stems off the GPU in wire format
-(clip prevention + PCM quantisation as device kernels).  File decoding still needs ``torchaudio``.
+(clip prevention + PCM quantisation as device kernels).  ``separate_audio_file`` decodes RIFF/WAVE files on the
+device (``demucs_b200.audio.load_audio``) and separates them there; other files still go through ``torchaudio``.
 """
 from __future__ import annotations
 
@@ -111,11 +112,21 @@ class Separator:
         self._samplerate = self._model.samplerate
 
     def _load_audio(self, track: Path):
+        """The reference's ``_load_audio`` with the device WAV decoder in place of ffmpeg: a RIFF/WAVE file comes back on
+        ``self._device`` at the model's rate and channel count; anything it cannot decode goes to torchaudio."""
+        from .audio import load_audio
+        errors = {}
+        try:
+            return load_audio(track, self._samplerate, self._audio_channels, device=self._device)[0]
+        except Exception as err:  # noqa
+            errors["demucs_b200.audio.load_audio"] = err
         try:
             import torchaudio as ta
             wav, sr = ta.load(str(track))
         except Exception as err:  # noqa
-            raise LoadAudioError(f"When trying to load using torchaudio, got the following error: {err}")
+            errors["torchaudio"] = err
+            raise LoadAudioError("\n".join(f"When trying to load using {backend}, got the following error: {error}"
+                                           for backend, error in errors.items()))
         if sr != self._samplerate or wav.shape[0] != self._audio_channels:      # api.py:221: convert_audio, on the device
             from .audio import convert_audio
             wav = convert_audio(wav.to(self._device), sr, self._samplerate, self._audio_channels).cpu()
@@ -164,7 +175,10 @@ class Separator:
         return {name: stems_to_pcm(stem, clip, bits_per_sample, as_float) for name, stem in stems.items()}
 
     def separate_audio_file(self, file: Path):
-        return self.separate_tensor(self._load_audio(file), self.samplerate)
+        """As the reference: ``(wav, {stem: tensor})`` on the host.  A WAV file is decoded, converted and
+        separated on the device; the wave and the stems come to the host at the end."""
+        wav, stems = self.separate_tensor(self._load_audio(file), self.samplerate)
+        return wav.cpu(), {name: stem.cpu() for name, stem in stems.items()}
 
     @property
     def samplerate(self):

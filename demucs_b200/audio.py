@@ -9,12 +9,15 @@ CPU tensors raise ``KernelError`` (use the reference, or move the tensor to the 
 ``julius`` is a third-party dependency that is not vendored in the reference tree (requirements.txt: julius>=0.2.3)
 and not installed here; the filter bank below restates its published algorithm (julius/resample.py, ResampleFrac:
 zeros=24, rolloff=0.945, Hann-windowed sinc, every phase normalised to unit sum, replicate padding, floor output
-length) -- parity with julius itself is UNPINNED, see oracle/audio_oracle.py.  File decoding (ffmpeg / torchaudio)
-and mp3 / flac encoding stay outside; ``save_audio`` writes RIFF/WAVE itself.
+length) -- parity with julius itself is UNPINNED, see oracle/audio_oracle.py.  ``save_audio`` writes RIFF/WAVE itself,
+and ``load_audio`` reads it: the header is parsed on the host, the data chunk goes to the GPU in its own encoding and one
+kernel decodes, de-interleaves and converts its channels.  Other containers (mp3, flac, ...) and mp3 / flac encoding
+stay outside.
 """
 from __future__ import annotations
 
 import math
+import os
 import struct
 import typing as tp
 from pathlib import Path
@@ -185,3 +188,129 @@ def save_audio(wav: torch.Tensor, path: tp.Union[str, Path], samplerate: int, bi
     with open(path, "wb") as f:
         f.write(header)
         f.write(data)
+
+
+_PCM = {(1, 8): 1, (1, 16): 2, (1, 24): 3, (1, 32): 4, (3, 32): 5, (3, 64): 6}     # (format tag, bits) -> BD_PCM_*
+_TAG_NAMES = {2: "MS ADPCM", 6: "A-law", 7: "\u00b5-law", 0x11: "IMA ADPCM"}
+_CONTAINERS = {b"RIFX": "RIFX (big-endian RIFF)", b"RF64": "RF64", b"BW64": "BW64", b"riff": "Sony Wave64"}
+_GUID_TAIL = bytes.fromhex("000000001000800000aa00389b71")      # KSDATAFORMAT_SUBTYPE_* after the 2-byte format tag
+# Bytes of one pinned staging buffer (rounded down to whole frames) and how many of them are in flight: pinned memory
+# stays bounded whatever the file's size, and the file read of one chunk overlaps the copy and decode of the previous.
+_CHUNK_BYTES = 4 << 20
+_RING = 3
+
+
+class _WavData(tp.NamedTuple):
+    pcm: int            # BD_PCM_*
+    channels: int
+    samplerate: int
+    block: int          # bytes per frame
+    offset: int         # file offset of the first frame
+    frames: int
+
+
+def _wav_fmt(body: bytes) -> tp.Tuple[int, int, int, int]:
+    """The ``fmt `` chunk -> (BD_PCM_*, channels, sample rate, bytes per frame)."""
+    if len(body) < 16:
+        raise ValueError(f"fmt chunk of {len(body)} bytes (at least 16 expected)")
+    tag, channels, samplerate, _, _, bits = struct.unpack("<HHIIHH", body[:16])
+    if tag == 0xFFFE:           # WAVE_FORMAT_EXTENSIBLE: the real tag heads the sub-format GUID; wValidBitsPerSample is
+        if len(body) < 40:      # ignored, samples are scaled by their container size (as ffmpeg does)
+            raise ValueError(f"WAVE_FORMAT_EXTENSIBLE fmt chunk of {len(body)} bytes (40 expected)")
+        if body[26:40] != _GUID_TAIL:
+            raise ValueError("WAVE_FORMAT_EXTENSIBLE with a sub-format GUID that is not a WAVE format tag")
+        tag = struct.unpack("<H", body[24:26])[0]
+    if tag not in (1, 3):
+        name = _TAG_NAMES.get(tag, "unsupported")
+        raise ValueError(f"WAVE format tag 0x{tag:04x} ({name}) is not decoded: PCM and IEEE float only")
+    if channels == 0:
+        raise ValueError("the fmt chunk declares zero channels")
+    if (tag, bits) not in _PCM:
+        kind = "integer PCM: 8, 16, 24 or 32" if tag == 1 else "IEEE float: 32 or 64"
+        raise ValueError(f"{bits} bits per sample is not decoded ({kind} bits)")
+    if samplerate == 0:
+        raise ValueError("the fmt chunk declares a sample rate of 0")
+    return _PCM[(tag, bits)], channels, samplerate, channels * bits // 8
+
+
+def _wav_layout(f: tp.BinaryIO, size: int) -> _WavData:
+    """Walks the RIFF chunks up to ``data``: chunks of other ids are skipped with their pad byte; a data size of 0,
+    0xFFFFFFFF or past the end of the file (streaming encoders) means the bytes present; a partial last frame is
+    dropped."""
+    head = f.read(12)
+    if head[:4] in _CONTAINERS:
+        raise ValueError(f"{_CONTAINERS[head[:4]]} files are not decoded: little-endian RIFF/WAVE only")
+    if len(head) < 12 or head[:4] != b"RIFF" or head[8:12] != b"WAVE":
+        raise ValueError("not a RIFF/WAVE file")
+    fmt = None
+    pos = 12
+    while True:
+        f.seek(pos)
+        ck = f.read(8)
+        if len(ck) < 8:
+            break
+        cid, n = ck[:4], struct.unpack("<I", ck[4:])[0]
+        if cid == b"fmt ":
+            fmt = _wav_fmt(f.read(n))
+        elif cid == b"data":
+            if fmt is None:
+                break
+            pcm, channels, samplerate, block = fmt
+            avail = size - (pos + 8)
+            frames = (n if 0 < n <= avail else avail) // block
+            if frames == 0:
+                raise ValueError("the data chunk holds no complete frame")
+            return _WavData(pcm, channels, samplerate, block, pos + 8, frames)
+        pos += 8 + n + (n & 1)
+    raise ValueError("no fmt chunk before the data chunk" if fmt is None else "no data chunk")
+
+
+def _read_into(f: tp.BinaryIO, buf: memoryview) -> None:
+    got = 0
+    while got < len(buf):
+        n = f.readinto(buf[got:])
+        if not n:
+            raise ValueError("the file ended inside its data chunk")
+        got += n
+
+
+def load_audio(path: tp.Union[str, Path], samplerate: tp.Optional[int] = None, channels: tp.Optional[int] = None,
+               device: tp.Union[str, torch.device] = "cuda") -> tp.Tuple[torch.Tensor, int]:
+    """A RIFF/WAVE file -> (wav [channels, length] float32 on ``device``, its sample rate).
+
+    Integer PCM (8 bit unsigned, 16 / 24 / 32 bit signed) and IEEE float (32 / 64 bit), plain or
+    WAVE_FORMAT_EXTENSIBLE, scaled to [-1, 1) as ``torchaudio.load(normalize=True)`` and ffmpeg do.  The data chunk
+    crosses PCIe in its own encoding (a 16-bit file at half the bytes of float) through a small ring of pinned buffers,
+    and ``bd_pcm_decode`` de-interleaves and scales it on the device.  ``channels``: convert as
+    ``convert_audio_channels`` does, in the same kernel.  ``samplerate``: resample with ``convert_audio`` (and return
+    that rate).  Other containers and codecs (RF64, A-law, ADPCM, ...) raise ``ValueError`` naming the reason."""
+    device = torch.device(device)
+    with open(path, "rb") as f:
+        info = _wav_layout(f, os.fstat(f.fileno()).st_size)
+        dst_ch = info.channels if channels is None else int(channels)
+        if dst_ch < 1 or not (dst_ch == info.channels or dst_ch == 1 or info.channels == 1 or info.channels >= dst_ch):
+            raise ValueError('The audio file has less channels than requested but is not mono.')
+        wav = torch.empty(dst_ch, info.frames, dtype=torch.float32, device=device)
+        _require_cuda(wav, "load_audio")
+        on_cuda = device.type == "cuda"
+        total = info.frames * info.block
+        chunk = min(max(_CHUNK_BYTES // info.block, 1) * info.block, total)
+        host = [torch.empty(chunk, dtype=torch.uint8, pin_memory=on_cuda) for _ in range(min(_RING, -(-total // chunk)))]
+        copied: tp.List[tp.Optional[torch.cuda.Event]] = [None] * len(host)
+        staged = torch.empty(chunk, dtype=torch.uint8, device=device)   # copy i + 1 follows decode i on the stream
+        f.seek(info.offset)
+        with torch.cuda.device(device) if on_cuda else _null():
+            for i, off in enumerate(range(0, total, chunk)):
+                slot = i % len(host)
+                if copied[slot] is not None:
+                    copied[slot].synchronize()          # the copy that last read this buffer has finished
+                n = min(chunk, total - off)
+                _read_into(f, memoryview(host[slot].numpy())[:n])
+                staged[:n].copy_(host[slot][:n], non_blocking=on_cuda)
+                if on_cuda:
+                    copied[slot] = torch.cuda.current_stream(device).record_event()
+                _lib.call("bd_pcm_decode", ptr(staged), ptr(wav), info.pcm, info.channels, dst_ch, n // info.block,
+                          info.frames, off // info.block, _stream(wav))
+    if samplerate is not None and samplerate != info.samplerate:
+        return convert_audio(wav, info.samplerate, samplerate, dst_ch), samplerate
+    return wav, info.samplerate

@@ -38,7 +38,7 @@ long long bd_attention_b16_ws_floats(int B, int H, int Tq, int Tk, int math);
 extern "C" {
 
 const char* bd_last_error(void) { return g_err; }
-int bd_version(void) { return 3; }   // 3: bf16-operand arithmetic (BD_MATH_BF16X3 / BD_MATH_BF16), gather / PCM entry points
+int bd_version(void) { return 4; }   // 4: bd_pcm_decode (WAV input decoded on the device); 3: bf16-operand arithmetic, gather / PCM entry points
 
 int bd_conv_gemm(const bd_gemm_desc* d, void* stream) {
   if (!d) {

@@ -260,6 +260,15 @@ int bd_absmax(const float* x, float* peak, long long n, void* stream);
 enum { BD_CLIP_NONE = 0, BD_CLIP_RESCALE = 1, BD_CLIP_CLAMP = 2, BD_CLIP_TANH = 3 };
 int bd_clip_pcm(const float* x, void* out, int channels, long long frames, int mode, const float* peak, int bits,
                 void* stream);
+/* The input side of the same wire format: src [frames, src_ch] interleaved little-endian PCM samples (the bytes of a
+ * WAV file's data chunk) -> dst[c * dst_ld + frame0 + t], t < frames, c < dst_ch (planar float; frame0 / dst_ld let
+ * the chunks of a long file land in one tensor).  Scaling as torchaudio.load(normalize=True) / ffmpeg's f32 output:
+ * u8 (x - 128) / 2^7, s16 x / 2^15, packed 3-byte s24 x / 2^23, s32 float_rn(x) / 2^31, f32 as is, f64 rounded to
+ * f32.  The channel rule is bd_convert_channels' (the mono down-mix summed in channel order, then divided by src_ch).
+ * src is aligned to the sample size (any alignment for s24); a frame is at most 32768 bytes. */
+enum { BD_PCM_U8 = 1, BD_PCM_S16 = 2, BD_PCM_S24 = 3, BD_PCM_S32 = 4, BD_PCM_F32 = 5, BD_PCM_F64 = 6 };
+int bd_pcm_decode(const void* src, float* dst, int format, int src_ch, int dst_ch, long long frames, long long dst_ld,
+                  long long frame0, void* stream);
 
 #ifdef __cplusplus
 }
