@@ -151,6 +151,8 @@ int bd_attention_simt(const float* q, const float* k, const float* v, float* o, 
                       int ldk, int ldv, int ldo, void* stream) {
   BD_REQUIRE(B > 0 && H > 0 && Tq > 0 && Tk > 0, "bd_attention: bad sizes");
   BD_REQUIRE(ldq % 4 == 0 && ldk % 4 == 0 && ldv % 4 == 0 && ldo % 4 == 0, "bd_attention: leading dims must be multiples of 4");
+  // every row is read and written as float4
+  BD_REQUIRE((((uintptr_t)q | (uintptr_t)k | (uintptr_t)v | (uintptr_t)o) & 15) == 0, "bd_attention: unaligned tensor");
   cudaError_t e = cudaFuncSetAttribute(attention_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM);
   if (e != cudaSuccess) {
     bd_set_error("bd_attention: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));

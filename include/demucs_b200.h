@@ -186,7 +186,8 @@ int bd_group_norm_apply(float* x, const float* mean_rstd, const float* gamma, co
                         long long rows_per_item, int C, void* stream);
 
 /* K6 (nn.MultiheadAttention via _sa_block/_ca_block, transformer.py:365,418,506): softmax(QK^T/8)V,
- * head_dim 64, no mask.  q [B,Tq,ldq] / k,v [B,Tk,ldk] / o [B,Tq,ldo]; head h uses columns [64h, 64h+64). */
+ * head_dim 64, no mask.  q [B,Tq,ldq] / k,v [B,Tk,ldk] / o [B,Tq,ldo]; head h uses columns [64h, 64h+64).
+ * Every arm: pointers 16-byte aligned, leading dims multiples of 4 (of 8 for bd_attention_bf16). */
 /* ws: workspace of bd_attention_workspace(...) floats for the tensor-core arms (V^T staging; hi/lo operand
  * splits for BD_MATH_TF32X3), may be NULL when that is 0 (BD_MATH_FP32). */
 long long bd_attention_workspace(int B, int H, int Tq, int Tk, int math);
